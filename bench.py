@@ -7,7 +7,7 @@ configs[2] ("c3"): 6 M splats, 1920x1080, 1-degree-per-frame orbit (the configur
 ">= 60 fps on a 6 M-splat scene @1080p on 1xB200" is quoted on).  N > 1 GPUs: screen-tile-row bands, one NCCL
 gather of the framebuffer per frame (strong scaling: the frame is fixed, the GPUs split it).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4] [--impl gsr|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4] [--impl gsr|reference] [--dump-outputs DIR]
 
 `--impl reference` times the CPU restatement of the reference pipeline (oracle/, all host threads) -- the
 reference itself needs Godot 4.3 + a Vulkan device and cannot run on this box (BASELINE.md section 2).
@@ -27,6 +27,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only; nothing is cached into it
 
 WORKLOADS = {
     # name: (N splats, W, H, seed, orbit?)      BASELINE.json configs[1..3]
@@ -56,7 +57,32 @@ def parse_args():
                          "NVLink peer memory + 4-byte NCCL sync; 'nccl' = NCCL gather of the band framebuffers")
     ap.add_argument("--overlap", type=int, default=-1, choices=[-1, 0, 1],
                     help="front/back overlap of consecutive frames (gsr_debug_pipeline): -1 = the library's default (off)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame the last timed step computed to DIR/*.npy (float32), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.gpus != 1 or args.workload == "c5"):
+        ap.error("--dump-outputs: only for one GPU and the frame workloads (c2, c3, c4)")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, rgba):
+    """The RGBA32F frame a caller of the timed path receives, as DIR/rgba.npy.  A frame above 64 MB (c4) is replaced by a fixed
+    sample of its pixels: DIR/rgba_sample.npy (k, 4) and their flat pixel indices y * W + x, DIR/rgba_sample_pixel.npy (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    rgba = np.ascontiguousarray(rgba, dtype=np.float32)
+    if rgba.nbytes <= DUMP_LIMIT_BYTES:
+        np.save(os.path.join(out_dir, "rgba.npy"), rgba)
+        return
+    px = rgba.reshape(-1, 4)
+    k = (DUMP_LIMIT_BYTES - 4096) // (px.itemsize * 4 + 8)   # 4096: the two .npy headers
+    idx = np.sort(np.random.default_rng(0).choice(px.shape[0], size=k, replace=False))
+    np.save(os.path.join(out_dir, "rgba_sample.npy"), px[idx])
+    np.save(os.path.join(out_dir, "rgba_sample_pixel.npy"), idx.astype(np.float64))
 
 
 def frame_params(wl, n_frames, first=0):
@@ -228,10 +254,10 @@ def run_reference(args, wl, rank, world):
         return
     splat60 = oracle_scene(wl)
     frames = frame_params(wl, args.warmup + args.steps)
-    # untimed warm-up (page-in, thread pool, thread-count choice), then as many of the K frames as fit in ~150 s
+    # untimed warm-up (page-in, thread pool, thread-count choice), then the K timed frames
     tune_cpu_threads(wl, splat60, frames[0])
-    stride = 1
-    ms, stages, threads, info = cpu_reference_frames(wl, splat60, frames[args.warmup::stride][:args.steps], 150.0)
+    kept = []
+    ms, stages, threads, info = cpu_reference_frames(wl, splat60, frames[args.warmup:args.warmup + args.steps], math.inf, keep=kept)
     mean_ms = float(np.mean(ms))
     value = wl["n"] / 1e6 * 1000.0 / mean_ms
     ref_shaders = reference_shaders_sample(wl, splat60, frames[args.warmup])
@@ -248,6 +274,8 @@ def run_reference(args, wl, rank, world):
         "gpu_launches": 0,
     }
     emit(line)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, kept[0][2].rgba)
 
 
 def reference_shaders_sample(wl, splat60, frame, every=4):
@@ -258,7 +286,7 @@ def reference_shaders_sample(wl, splat60, frame, every=4):
         from oracle import oracle as orc
         from oracle import refshaders
         if not refshaders.available():
-            return {"unavailable": "oracle/_ref not built (no /root/reference in this container and no prebuilt libraries)"}
+            return {"unavailable": "oracle/_ref not built (GSR_REFERENCE_DIR did not name the original project at build time)"}
         sub = np.ascontiguousarray(splat60[::every])
         vp, ub = frame
         spec = orc.frame(sub, vp, orc.uniforms_from_bytes(np.frombuffer(ub, dtype=np.uint8)))
@@ -285,20 +313,21 @@ def run_c5(args):
     sizes = [20, 22, 24, 26, 28]
     res = {}
     for lg in sizes:
-        res[f"2^{lg}"] = radix_microbench(torch, 0, 1 << lg)
+        res[f"2^{lg}"] = radix_microbench(torch, 0, 1 << lg, steps=args.steps, warmup=args.warmup)
     top = res[f"2^{sizes[-1]}"]
     peak, peak_src = measured_peak_gbs()
-    emit({"metric": "Gkeys/s", "value": top["pairs"]["gkeys_s"], "unit": "Gpairs/s (32-bit key + 32-bit value)", "n_gpus": 1, "steps": 3, "warmup": 1,
+    emit({"metric": "Gkeys/s", "value": top["pairs"]["gkeys_s"], "unit": "Gpairs/s (32-bit key + 32-bit value)", "n_gpus": 1, "steps": args.steps, "warmup": args.warmup,
           "ms_per_step": top["pairs"]["ms"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u32", "data": "synthetic",
           "config": {"workload": "c5: " + WORKLOADS["c5"]["desc"], "sizes": res, "l2": "2^26 and 2^28 exceed L2; smaller sizes are L2-resident"},
           "roofline": {"kernel": "sort_hist_kernel + 4x onesweep_kernel", "bound": "hbm", "achieved": top["pairs"]["hbm_frac_of_measured"] * peak, "peak": peak,
                        "unit": "GB/s", "frac": top["pairs"]["hbm_frac_of_measured"], "traffic": None, "peak_source": peak_src,
                        "algorithmic_bytes": "68 B per pair (36 B per key keys-only), SURVEY 8d"},
-          "keys_only_gkeys_s": top["keys"]["gkeys_s"], "gpu_launches": 5 * 4 * 2 * len(sizes), "e2e": None, "cpu_baseline": None})
+          "keys_only_gkeys_s": top["keys"]["gkeys_s"], "gpu_launches": 5 * (args.warmup + args.steps) * 2 * len(sizes), "e2e": None, "cpu_baseline": None})
 
 
-def radix_microbench(torch, device_index, n=1 << 26):
-    """config c5 point: n (tile<<16|depth16) keys + u32 values, device resident, CUDA events on the sort stream."""
+def radix_microbench(torch, device_index, n=1 << 26, steps=3, warmup=1):
+    """config c5 point: n (tile<<16|depth16) keys + u32 values, device resident, CUDA events on the sort stream; mean of `steps`
+    timed sorts after `warmup` untimed ones."""
     import ctypes as C
     from godotgaussiansplatting_b200 import _lib
     from godotgaussiansplatting_b200.synthetic import radix_keys
@@ -311,7 +340,7 @@ def radix_microbench(torch, device_index, n=1 << 26):
     try:
         for name, with_vals in (("pairs", True), ("keys", False)):
             best = []
-            for it in range(4):
+            for it in range(warmup + steps):
                 k = keys.clone()
                 v = vals.clone() if with_vals else None
                 torch.cuda.synchronize()
@@ -320,7 +349,7 @@ def radix_microbench(torch, device_index, n=1 << 26):
                 torch.cuda.synchronize()
                 ms = C.c_float()
                 _lib.check(L.gsr_sorter_last_ms(s, C.byref(ms)), "ms")
-                if it:
+                if it >= warmup:
                     best.append(ms.value)
             t = float(np.mean(best))
             out[name] = {"n": n, "ms": t, "gkeys_s": n / t / 1e6, "hbm_frac_of_measured": (n * (68 if with_vals else 36) / (t * 1e-3)) / 1e9 / measured_peak_gbs()[0]}
@@ -524,6 +553,7 @@ def main():
     sampler = ClockSampler(torch.cuda.current_device() if "CUDA_VISIBLE_DEVICES" not in os.environ else local_rank) if rank == 0 else None
     total_ms = timed(e2e=False)
     clocks = sampler.stop() if sampler else None
+    last_frame = rast.read_framebuffer() if args.dump_outputs else None   # the frame of the last timed step (after the stream sync)
     hist = rast.frame_history(min(args.steps, 512))
     st = rast.stats()
     e2e_ms = timed(e2e="rgba")
@@ -670,6 +700,8 @@ def main():
             "reference_published": {"fps": 108, "scene": "bicycle.ply ~6.1M splats @1080p", "hw": "RTX 3060 Ti", "source": "README.md:58 (other hardware; not comparable)"},
         }
         emit(line)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_frame)
     rast.cleanup_gpu()
     if world > 1:
         dist.destroy_process_group()

@@ -1,7 +1,7 @@
 """Build oracle/_ref/libgsr_refshaders{,_libm}.so: the reference's six compute shaders compiled for the CPU.
 
-TEST INFRASTRUCTURE.  Recipe (the prompt's "compile the reference from the sources where they lie"):
-  /root/reference/resources/shaders/compute/*.glsl --translate.py--> C++ in a temporary directory
+TEST INFRASTRUCTURE.  Recipe (the reference compiled from the sources where they lie):
+  $GSR_REFERENCE_DIR/resources/shaders/compute/*.glsl --translate.py--> C++ in a temporary directory
   --g++ -ffp-contract=off, glsl_emu.hpp--> oracle/_ref/*.so        (git-ignored; travels to the GPU box)
 No reference source is written into the repository; the temporary C++ is deleted after the link.
 Two variants: exp()/pow() from the oracle's deterministic orc_exp/orc_pow (bit-exact comparisons with gsr_oracle.c),
@@ -18,7 +18,9 @@ import tempfile
 HERE = os.path.dirname(os.path.abspath(__file__))
 ORACLE_DIR = os.path.dirname(HERE)
 OUT_DIR = os.path.join(ORACLE_DIR, "_ref")
-REFERENCE_SHADERS = "/root/reference/resources/shaders/compute"
+# a checkout of the original project; without it only prebuilt libraries count (tests use tests/golden instead)
+REFERENCE_DIR = os.environ.get("GSR_REFERENCE_DIR", "")
+REFERENCE_SHADERS = os.path.join(REFERENCE_DIR, "resources", "shaders", "compute")
 SHADERS = ("gsplat_projection", "radix_sort_upsweep", "radix_sort_spine", "radix_sort_downsweep", "gsplat_boundaries",
            "gsplat_render")
 CXX = os.environ.get("ORC_CXX", "/usr/bin/g++")
@@ -30,11 +32,11 @@ def lib_path(libm: bool = False) -> str:
 
 
 def reference_available() -> bool:
-    return all(os.path.isfile(os.path.join(REFERENCE_SHADERS, s + ".glsl")) for s in SHADERS)
+    return bool(REFERENCE_DIR) and all(os.path.isfile(os.path.join(REFERENCE_SHADERS, s + ".glsl")) for s in SHADERS)
 
 
 def build(force: bool = False, verbose: bool = False) -> bool:
-    """Returns True when both libraries exist afterwards.  Without /root/reference only prebuilt files count."""
+    """Returns True when both libraries exist afterwards.  Without the reference only prebuilt files count."""
     have = os.path.isfile(lib_path(False)) and os.path.isfile(lib_path(True))
     if not reference_available():
         return have
@@ -76,4 +78,4 @@ def build(force: bool = False, verbose: bool = False) -> bool:
 
 if __name__ == "__main__":
     ok = build(force="--force" in sys.argv, verbose=True)
-    print("refshaders:", "built" if ok else "unavailable (no /root/reference and no prebuilt oracle/_ref)")
+    print("refshaders:", "built" if ok else "unavailable (GSR_REFERENCE_DIR unset and no prebuilt oracle/_ref)")

@@ -43,7 +43,7 @@ def available() -> bool:
 def _lib(libm: bool) -> C.CDLL:
     if libm not in _libs:
         if not _build_ref.build():
-            raise RuntimeError("oracle/_ref/libgsr_refshaders*.so missing and /root/reference not available to build it")
+            raise RuntimeError("oracle/_ref/libgsr_refshaders*.so missing and GSR_REFERENCE_DIR does not name the reference to build it")
         if not libm:
             from . import oracle as _oracle   # makes sure libgsr_oracle.so (orc_test_exp/pow) exists
             _oracle.build()

@@ -1,5 +1,5 @@
-"""Mints tests/golden/demo_subset.npz from the reference's only fixture, resources/demo.ply (run in the build
-container where /root/reference is mounted):  python tests/golden/make_golden.py
+"""Mints tests/golden/demo_subset.npz from the reference's only fixture, resources/demo.ply, with a checkout of the original
+project:  GSR_REFERENCE_DIR=<original project> python tests/golden/make_golden.py
 
 Contents: every 33rd splat of demo.ply (8216 vertices, the raw 62 floats each), the default camera of
 util/camera.gd:151-153 at 320x240, and for that frame
@@ -7,7 +7,7 @@ util/camera.gd:151-153 at 320x240, and for that frame
               oracle/_ref/libgsr_refshaders.so): M, sorted keys/values, tile ranges, the rgba32f texture;
   * keys/values/bounds/rgba -- the oracle's outputs under the gsr spec (identical integers; pixels differ from ref_rgba
               only by the spec's five explicit FMA contractions, <= 1e-4).
-The vectors travel to the GPU box, where /root/reference does not exist.
+The tests need only the stored vectors, not the original project.
 """
 import os
 import sys
@@ -21,7 +21,7 @@ from godotgaussiansplatting_b200.ply_file import PlyFile, swizzle_splats  # noqa
 from oracle import oracle as orc  # noqa: E402
 from tests.scenes import uniforms_bytes  # noqa: E402
 
-ply = PlyFile("/root/reference/resources/demo.ply")
+ply = PlyFile(os.path.join(os.environ["GSR_REFERENCE_DIR"], "resources", "demo.ply"))
 sub = np.ascontiguousarray(ply.table[::33])
 W, H = 320, 240
 c = cam.default_camera(aspect=W / H)

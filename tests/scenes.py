@@ -27,3 +27,16 @@ def uniforms_bytes(cam_pos, model_scale, width, height, time) -> bytes:
     raw = bytearray(buf.tobytes())
     raw[16:24] = np.array([width, height], dtype=np.int32).tobytes()
     return bytes(raw)
+
+
+def demo_subset_scene():
+    """Every 33rd splat of the original project's resources/demo.ply (tests/golden/demo_subset.npz, 8216 splats) through the
+    ingest restatement of the oracle, at the reference's default camera, 640x480.  Returns (ply62, splat60, vp32, uniforms_bytes)."""
+    import os
+
+    from oracle import oracle as orc
+    with np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "demo_subset.npz")) as g:
+        ply62 = g["ply62"]
+    c = cam.default_camera(aspect=640 / 480)
+    vp = cam.pack_camera_push_constants(c.get_camera_transform(), c.get_camera_projection())
+    return ply62, orc.preprocess_ply(ply62, 0.0), vp, uniforms_bytes([0.0, 0.0, 0.0], 1.0, 640, 480, 10.0)

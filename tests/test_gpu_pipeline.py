@@ -494,7 +494,7 @@ def test_presentation_formats_match_the_oracle_frame_through_the_same_conversion
 def test_uncontracted_blend_flag_is_bit_identical_to_the_reference_shader_text():
     """GSR_FLAG_UNCONTRACTED_BLEND (VERDICT r01 weak #3): with no fma contraction anywhere in gsplat_render.glsl:84-90 the GPU frame is
     bit-identical to the oracle's uncontracted evaluation -- the evaluation the reference's own shader text gives when it is executed
-    on the CPU (oracle/_ref; compared directly when the prebuilt reference-shader library is present)."""
+    on the CPU (its frame's digest is stored in tests/golden/refshaders.json)."""
     n, w, h = 30000, 640, 360
     splat60, vp, ub = make_scene(n, 23, w, h, scale_boost=0.8)
     u = orc.uniforms_from_bytes(np.frombuffer(ub, dtype=np.uint8))
@@ -511,11 +511,5 @@ def test_uncontracted_blend_flag_is_bit_identical_to_the_reference_shader_text()
     np.testing.assert_array_equal(t["keys"], ref.keys)
     np.testing.assert_array_equal(bits(img), bits(ref.rgba))
     assert float(np.abs(img - spec.rgba).max()) <= 1e-4 and not np.array_equal(bits(img), bits(spec.rgba))   # a different member of the legal set
-    try:
-        from oracle import refshaders
-        if refshaders.available():
-            refshaders.set_shared_fill(int(ref.keys[0] >> 16))
-            rf = refshaders.ReferencePipeline(splat60, w, h).rasterize(vp, ub)
-            np.testing.assert_array_equal(bits(img), bits(rf.rgba))
-    except (OSError, RuntimeError):
-        pass
+    from tests.refgolden import digest, golden
+    assert digest(img) == golden("uncontracted_blend")["rgba"], "frame differs from the reference shaders' frame"

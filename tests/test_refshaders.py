@@ -3,6 +3,9 @@
 oracle/_ref/libgsr_refshaders.so is the six .glsl files of the reference compiled for the CPU (oracle/glsl_cpu:
 declarations rewrapped, every statement and expression the shader author's; workgroups as fibers with real barriers and
 32-wide subgroup collectives).  oracle/refshaders.py issues the dispatches of `rasterize()` (rasterizer.gd:122-160).
+What those shaders computed for every case below is stored under tests/golden (tests/refgolden.py; minted by
+tests/golden/make_refshaders_golden.py from the builders in this module), so the comparison needs neither the reference
+nor oracle/_ref.
 
 What is asserted
   * projection: the 48-byte records, the emitted (key, value) pairs and M are bit-identical to gsr_oracle.c;
@@ -11,16 +14,13 @@ What is asserted
   * pixels: bit-identical to the oracle's uncontracted evaluation, and within the north-star 1e-4 of the gsr spec (the five
     explicit contractions the CUDA compositor uses) -- both are legal evaluations of the GLSL text;
   * (-m gpu) the CUDA frame through the C-ABI against the reference-shader frame directly.
-The libraries are built here when /root/reference is present and travel prebuilt (git-ignored) to the GPU box.
 """
 import numpy as np
 import pytest
 
 from oracle import oracle as orc
-from oracle import refshaders
-from tests.scenes import make_scene
-
-pytestmark = pytest.mark.skipif(not refshaders.available(), reason="oracle/_ref not built and /root/reference absent")
+from tests.refgolden import LIBM_STEP, bits, digest, golden, libm_delta
+from tests.scenes import demo_subset_scene, make_scene
 
 RGBA_TOL = 1e-4
 
@@ -32,93 +32,30 @@ SCENES = {
     "scaled_heatmap": (8000, 9, 224, 128, 120, 10.0, 0.5, 1.0, 0.0, 1.5),
     "three_splats": (3, 11, 64, 48, None, 10.0, 1.0, 0.0, 0.0, 2.0),
 }
+RAGGED = [(1, 1), (2, 3), (15, 15), (16, 16), (17, 17), (31, 33), (257, 1), (640, 16)]
+SPLAT_COUNTS = [1, 2, 33, 257]
+FUZZ = [(123, 11), (321, 200)]
+SORT_SIZES = [1, 2, 255, 4095, 4096, 4097, 12289, 50000]
 
 
-def bits(a):
-    return np.ascontiguousarray(a).view(np.uint32)
-
-
+# ---------------------------------------------------------------- inputs (shared with tests/golden/make_refshaders_golden.py)
 def build(name):
     n, seed, w, h, frame, time, ms, heat, creation, boost = SCENES[name]
     splat60, vp, ub = make_scene(n, seed, w, h, frame=frame, time=time, model_scale=ms, creation_time=creation, scale_boost=boost)
     return splat60, vp, ub, w, h, heat
 
 
-def reference_frame(splat60, vp, ub, w, h, heat, first_tile, libm=False, target_tile=-1):
-    # the shared word gsplat_boundaries.glsl:36 reads uninitialised (Q20) holds the first key's tile: the author's intent
-    refshaders.set_shared_fill(first_tile, libm=libm)
-    return refshaders.ReferencePipeline(splat60, w, h, libm=libm).rasterize(vp, ub, heatmap=heat, target_tile=target_tile)
-
-
-def oracle_frames(splat60, vp, ub, heat):
-    u = orc.uniforms_from_bytes(np.frombuffer(ub, dtype=np.uint8))
-    spec = orc.frame(splat60, vp, u, heatmap=heat)
-    orc.set_blend_contraction(False)
-    try:
-        strict = orc.frame(splat60, vp, u, heatmap=heat)
-    finally:
-        orc.set_blend_contraction(True)
-    return spec, strict, u
-
-
-def assert_stages_equal(ref, spec, splat60, vp, u):
-    """ref: ReferenceFrame from the shaders; spec: oracle Frame."""
-    assert not spec.overflow
-    assert ref.duplicates == spec.duplicates
-    pr = orc.project(splat60, vp, u)
-    np.testing.assert_array_equal(ref.keys_unsorted, pr.keys)
-    np.testing.assert_array_equal(ref.values_unsorted, pr.values)
-    vis = np.unique(pr.values)
-    assert vis.size == spec.visible
-    for f in orc.RECORD_DTYPE.names:
-        np.testing.assert_array_equal(bits(ref.records[f][vis]), bits(pr.records[f][vis]), err_msg=f"record field {f}")
-    np.testing.assert_array_equal(ref.keys, spec.keys)
-    np.testing.assert_array_equal(ref.values, spec.values)
-    np.testing.assert_array_equal(ref.bounds, spec.bounds)
-    m = spec.duplicates
-    assert ref.grid_dims[0] == max(1, -(-m // 4096)) and ref.grid_dims[3] == max(1, -(-m // 256))   # :212-213
-
-
-@pytest.mark.parametrize("name", list(SCENES))
-def test_reference_shaders_equal_oracle_bit_for_bit(name):
-    splat60, vp, ub, w, h, heat = build(name)
-    spec, strict, u = oracle_frames(splat60, vp, ub, heat)
-    assert spec.duplicates > 0
-    ref = reference_frame(splat60, vp, ub, w, h, heat, int(spec.keys[0] >> 16))
-    assert_stages_equal(ref, spec, splat60, vp, u)
-    # pixels: the shader text without contraction == the oracle without contraction, bit for bit ...
-    np.testing.assert_array_equal(bits(ref.rgba), bits(strict.rgba))
-    # ... and the gsr spec (explicit contractions, what libgsr computes) is inside the north-star tolerance of it
-    assert np.abs(ref.rgba - spec.rgba).max() <= RGBA_TOL
-    assert np.all(ref.rgba[..., 3] == 1.0)
-
-
-def check_scene(splat60, vp, ub, w, h, heat=0.0):
-    spec, strict, u = oracle_frames(splat60, vp, ub, heat)
-    first = int(spec.keys[0] >> 16) if spec.duplicates else 0
-    ref = reference_frame(splat60, vp, ub, w, h, heat, first)
-    assert_stages_equal(ref, spec, splat60, vp, u)
-    np.testing.assert_array_equal(bits(ref.rgba), bits(strict.rgba))
-    assert np.abs(ref.rgba - spec.rgba).max() <= RGBA_TOL
-    return ref, spec
-
-
-@pytest.mark.parametrize("w,h", [(1, 1), (2, 3), (15, 15), (16, 16), (17, 17), (31, 33), (257, 1), (640, 16)])
-def test_ragged_resolutions(w, h):
-    """Partial tiles: off-image invocations still vote in the tile-stop rule (Q9/Q17) and imageStore drops their texels."""
+def ragged_scene(w, h):
     splat60, vp, ub = make_scene(3000, 50, w, h, scale_boost=1.0)
-    check_scene(splat60, vp, ub, w, h)
+    return splat60, vp, ub, w, h, 0.0
 
 
-@pytest.mark.parametrize("n", [1, 2, 33, 257])
-def test_splat_counts_around_subgroup_and_workgroup_sizes(n):
+def splat_count_scene(n):
     splat60, vp, ub = make_scene(n, 60 + n, 320, 240, scale_boost=-1.5)   # capacity is the static 10 n (Q12): keep M below it
-    check_scene(splat60, vp, ub, 320, 240)
+    return splat60, vp, ub, 320, 240, 0.0
 
 
-def test_one_splat_covering_every_tile_hits_the_last_grid_tile_rule():
-    """A splat whose rect is the whole grid: the last occupied tile IS tile T-1, so gsplat_boundaries.glsl:47-49 stores
-    M-1 as its end (Q10: the final instance of the last grid tile is dropped)."""
+def one_splat_covering_every_tile_scene():
     w, h, n = 640, 480, 200                       # cap = 10 n = 2000 >= the 1200 tiles
     splat60, vp, ub = make_scene(n, 70, w, h)
     splat60[:, 0:3] = (0.0, 0.0, 2.5)
@@ -126,29 +63,20 @@ def test_one_splat_covering_every_tile_hits_the_last_grid_tile_rule():
     splat60[0, 4], splat60[0, 7], splat60[0, 9] = 4.0, 4.0, 4.0
     splat60[1:, 4], splat60[1:, 7], splat60[1:, 9] = 1e-6, 1e-6, 1e-6
     splat60[:, 10] = 0.5
-    ref, spec = check_scene(splat60, vp, ub, w, h)
-    T = ref.bounds.shape[0]
-    assert spec.duplicates >= T and int(ref.keys[-1] >> 16) == T - 1
-    assert ref.bounds[T - 1, 1] == spec.duplicates - 1
+    return splat60, vp, ub, w, h, 0.0
 
 
-def test_everything_culled():
-    """M = 0: the sort runs on one empty partition, no range is written, the frame is black with alpha 1."""
+def everything_culled_scene():
     w, h, n = 160, 96, 500
     splat60, vp, ub = make_scene(n, 90, w, h)
     splat60[:, 2] = -np.abs(splat60[:, 2]) - 50.0     # behind the camera / outside the frustum
-    spec, _, u = oracle_frames(splat60, vp, ub, 0.0)
+    spec, _, _ = oracle_frames(splat60, vp, ub, 0.0)
     if spec.duplicates:                                  # the camera looks down the other axis: flip
         splat60[:, 2] = -splat60[:, 2]
-        spec, _, u = oracle_frames(splat60, vp, ub, 0.0)
-    assert spec.duplicates == 0
-    ref = reference_frame(splat60, vp, ub, w, h, 0.0, 0)
-    assert ref.duplicates == 0 and not ref.bounds.any()
-    np.testing.assert_array_equal(bits(ref.rgba), bits(spec.rgba))
-    assert not ref.rgba[..., :3].any() and np.all(ref.rgba[..., 3] == 1.0)
+    return splat60, vp, ub, w, h, 0.0
 
 
-def test_degenerate_splats():
+def degenerate_scene():
     """opacity 0 (pow(0, .2) = 0 -> radius 0), zero covariance (only the +0.3 dilation), opacity logit extremes."""
     n, w, h = 2000, 320, 240
     splat60, vp, ub = make_scene(n, 80, w, h, scale_boost=1.0)
@@ -156,8 +84,7 @@ def test_degenerate_splats():
     splat60[9, 4:10] = 0.0
     splat60[10, 10] = 1.0
     splat60[11, 10] = 1e-30
-    ref, spec = check_scene(splat60, vp, ub, w, h)
-    assert (ref.values == 8).sum() <= 1          # radius 0 still rounds out to the one tile under the centre
+    return splat60, vp, ub, w, h, 0.0
 
 
 def adversarial_splats(n, seed, w, h, frame):
@@ -183,35 +110,19 @@ def adversarial_splats(n, seed, w, h, frame):
     return splat60, vp, ub
 
 
-@pytest.mark.parametrize("seed,frame", [(123, 11), (321, 200)])
-def test_projection_fuzz(seed, frame):
-    """gsplat_projection.glsl alone on adversarial splats: M, every emitted pair and every record bit for bit."""
+def projection_fuzz_scene(seed, frame):
     n, w, h = 100000, 640, 360
     splat60, vp, ub = adversarial_splats(n, seed, w, h, frame)
     splat60[30000:, 0:3] = 1e9        # 70 000 culled fillers: the reference sizes the pair buffers as 10 x point count (Q12)
-    u = orc.uniforms_from_bytes(np.frombuffer(ub, dtype=np.uint8))
-    pr = orc.project(splat60, vp, u, cap=10 * n)
-    assert 0 < pr.duplicates <= 10 * n and pr.visible > 500
-    P = refshaders.ReferencePipeline(splat60, w, h)
-    P.uniforms[:] = np.frombuffer(bytes(ub), dtype=np.float32)
-    P.histogram[: 1 + 4 * refshaders.RADIX] = 0
-    P._dispatch("gsplat_projection", ((n + 255) // 256, 1, 1),
-                [P.splats, P.culled, P.histogram, P.sort_keys, P.sort_values, P.grid_dims, P.uniforms], np.asarray(vp, dtype=np.float32).tobytes())
-    assert int(P.histogram[0]) == pr.duplicates
-    np.testing.assert_array_equal(P.sort_keys[: pr.duplicates], pr.keys)
-    np.testing.assert_array_equal(P.sort_values[: pr.duplicates], pr.values)
-    vis = np.unique(pr.values)
-    for f in orc.RECORD_DTYPE.names:
-        np.testing.assert_array_equal(bits(P.culled[f][vis]), bits(pr.records[f][vis]), err_msg=f"record field {f}")
+    return splat60, vp, ub, w, h
 
 
-def test_render_fuzz():
-    """gsplat_render.glsl alone on synthetic records and ranges: indefinite conics (positive power, alpha > 1, negative
-    transmittance -- Q8: nothing is clamped), ranges that run past their chunk, the heat-map term."""
+def render_fuzz_inputs():
+    """Synthetic records and ranges: indefinite conics (positive power, alpha > 1, negative transmittance -- Q8: nothing is
+    clamped), ranges that run past their chunk, the heat-map term.  Returns (records, values, bounds, w, h)."""
     rng = np.random.default_rng(77)
     w, h, nrec = 96, 64, 5000
-    gx, gy = (w + 15) // 16, (h + 15) // 16
-    T = gx * gy
+    T = ((w + 15) // 16) * ((h + 15) // 16)
     rec = np.zeros(nrec, dtype=orc.RECORD_DTYPE)
     rec["image_pos"] = rng.uniform(-20, [w + 20, h + 20], (nrec, 2)).astype(np.float32)
     rec["conic"] = np.stack([rng.uniform(-0.002, 0.05, nrec), rng.uniform(-0.03, 0.03, nrec), rng.uniform(-0.002, 0.05, nrec)], axis=1).astype(np.float32)
@@ -225,43 +136,148 @@ def test_render_fuzz():
     bounds[:, 0] = np.concatenate([[0], np.cumsum(lens)[:-1]])
     bounds[:, 1] = bounds[:, 0] + lens
     bounds[3] = (50, 10)                                                # end < start: max(0, int(y - x)) = 0 splats (:61)
+    return rec, values, bounds, w, h
+
+
+def boundaries_garbage_words(spec):
+    """Values for the shared word gsplat_boundaries.glsl:36 reads uninitialised (Q20); the last is the first key's tile."""
+    first = int(spec.keys[0] >> 16)
+    return (0xFFFFFFFF, 0, first + 1, spec.bounds.shape[0] - 1, first)
+
+
+def sort_inputs(n):
+    rng = np.random.default_rng(n)
+    keys = rng.integers(0, 2**32, n, dtype=np.uint64).astype(np.uint32)
+    if n > 1000:
+        keys[: n // 2] = keys[: n // 2] & np.uint32(0xFFFF00FF)       # many ties: stability is observable
+    return keys, np.arange(n, dtype=np.uint32)
+
+
+def pick_target_tile(spec):
+    counts = spec.bounds[:, 1].astype(np.int64) - spec.bounds[:, 0].astype(np.int64)
+    return int(np.argmax(counts)), counts
+
+
+def demo_scene():
+    _, s, vp, ub = demo_subset_scene()
+    return s, vp, ub, 640, 480, 0.0
+
+
+def oracle_frames(splat60, vp, ub, heat):
+    u = orc.uniforms_from_bytes(np.frombuffer(ub, dtype=np.uint8))
+    spec = orc.frame(splat60, vp, u, heatmap=heat)
+    orc.set_blend_contraction(False)
+    try:
+        strict = orc.frame(splat60, vp, u, heatmap=heat)
+    finally:
+        orc.set_blend_contraction(True)
+    return spec, strict, u
+
+
+# ---------------------------------------------------------------- checks against the stored reference outputs
+def assert_stages_equal(ref, spec, strict, splat60, vp, u):
+    """ref: golden record of the reference shaders' frame; spec / strict: oracle Frames with / without the spec's contractions."""
+    assert not spec.overflow
+    assert ref["duplicates"] == spec.duplicates
+    pr = orc.project(splat60, vp, u)
+    assert digest(pr.keys) == ref["keys_unsorted"], "emitted keys differ from the reference shaders"
+    assert digest(pr.values) == ref["values_unsorted"], "emitted values differ from the reference shaders"
+    vis = np.unique(pr.values)
+    assert vis.size == spec.visible
+    assert digest(pr.records[vis]) == ref["records"], "records of the visible splats differ from the reference shaders"
+    assert digest(spec.keys) == ref["keys"], "sorted keys differ from the reference shaders"
+    assert digest(spec.values) == ref["values"], "sorted values differ from the reference shaders"
+    assert digest(spec.bounds) == ref["bounds"], "tile ranges differ from the reference shaders"
+    m = spec.duplicates
+    assert ref["grid_dims"][0] == max(1, -(-m // 4096)) and ref["grid_dims"][3] == max(1, -(-m // 256))   # :212-213
+    # pixels: the shader text without contraction == the oracle without contraction, bit for bit ...
+    assert digest(strict.rgba) == ref["rgba"], "the oracle's uncontracted frame differs from the reference shaders' frame"
+
+
+def check_scene(case, splat60, vp, ub, w, h, heat=0.0):
+    """Returns the oracle's (spec, strict) frames; strict.rgba is the reference shaders' frame, bit for bit."""
+    spec, strict, u = oracle_frames(splat60, vp, ub, heat)
+    assert_stages_equal(golden(case), spec, strict, splat60, vp, u)
+    # ... and the gsr spec (explicit contractions, what libgsr computes) is inside the north-star tolerance of it
+    assert np.abs(strict.rgba - spec.rgba).max() <= RGBA_TOL
+    return spec, strict
+
+
+@pytest.mark.parametrize("name", list(SCENES))
+def test_reference_shaders_equal_oracle_bit_for_bit(name):
+    splat60, vp, ub, w, h, heat = build(name)
+    spec, strict = check_scene(f"scene/{name}", splat60, vp, ub, w, h, heat)
+    assert spec.duplicates > 0
+    assert np.all(strict.rgba[..., 3] == 1.0)
+
+
+@pytest.mark.parametrize("w,h", RAGGED)
+def test_ragged_resolutions(w, h):
+    """Partial tiles: off-image invocations still vote in the tile-stop rule (Q9/Q17) and imageStore drops their texels."""
+    check_scene(f"ragged/{w}x{h}", *ragged_scene(w, h))
+
+
+@pytest.mark.parametrize("n", SPLAT_COUNTS)
+def test_splat_counts_around_subgroup_and_workgroup_sizes(n):
+    check_scene(f"splats/{n}", *splat_count_scene(n))
+
+
+def test_one_splat_covering_every_tile_hits_the_last_grid_tile_rule():
+    """A splat whose rect is the whole grid: the last occupied tile IS tile T-1, so gsplat_boundaries.glsl:47-49 stores
+    M-1 as its end (Q10: the final instance of the last grid tile is dropped)."""
+    spec, _ = check_scene("one_splat_covering_every_tile", *one_splat_covering_every_tile_scene())
+    T = spec.bounds.shape[0]
+    assert spec.duplicates >= T and int(spec.keys[-1] >> 16) == T - 1
+    assert spec.bounds[T - 1, 1] == spec.duplicates - 1
+
+
+def test_everything_culled():
+    """M = 0: the sort runs on one empty partition, no range is written, the frame is black with alpha 1."""
+    splat60, vp, ub, w, h, heat = everything_culled_scene()
+    spec, _, _ = oracle_frames(splat60, vp, ub, heat)
+    assert spec.duplicates == 0
+    ref = golden("everything_culled")
+    assert ref["duplicates"] == 0 and digest(spec.bounds) == ref["bounds"] and not spec.bounds.any()
+    assert digest(spec.rgba) == ref["rgba"]
+    assert not spec.rgba[..., :3].any() and np.all(spec.rgba[..., 3] == 1.0)
+
+
+def test_degenerate_splats():
+    spec, _ = check_scene("degenerate_splats", *degenerate_scene())
+    assert (spec.values == 8).sum() <= 1          # radius 0 still rounds out to the one tile under the centre
+
+
+@pytest.mark.parametrize("seed,frame", FUZZ)
+def test_projection_fuzz(seed, frame):
+    """gsplat_projection.glsl alone on adversarial splats: M, every emitted pair and every record bit for bit."""
+    splat60, vp, ub, w, h = projection_fuzz_scene(seed, frame)
+    n = splat60.shape[0]
+    u = orc.uniforms_from_bytes(np.frombuffer(ub, dtype=np.uint8))
+    pr = orc.project(splat60, vp, u, cap=10 * n)
+    assert 0 < pr.duplicates <= 10 * n and pr.visible > 500
+    ref = golden(f"projection_fuzz/{seed}-{frame}")
+    assert ref["duplicates"] == pr.duplicates
+    assert digest(pr.keys) == ref["keys_unsorted"] and digest(pr.values) == ref["values_unsorted"]
+    assert digest(pr.records[np.unique(pr.values)]) == ref["records"]
+
+
+def test_render_fuzz():
+    """gsplat_render.glsl alone on synthetic records and ranges (render_fuzz_inputs)."""
+    rec, values, bounds, w, h = render_fuzz_inputs()
     orc.set_blend_contraction(False)
     try:
         want, _, _ = orc.render(rec, values, bounds, w, h, heatmap=1.0)
     finally:
         orc.set_blend_contraction(True)
-    refshaders.set_shared_fill(0)
-    L = refshaders._lib(False)
-    tex = np.zeros((h, w, 4), dtype=np.float32)
-    pick = np.zeros(4, dtype=np.float32)
-    bufs = [rec, values, bounds, pick, tex]
-    import ctypes as C
-    ptrs = (C.c_void_p * 5)(*[b.ctypes.data for b in bufs])
-    sizes = (C.c_size_t * 5)(*[b.nbytes for b in bufs])
-    push = C.create_string_buffer(refshaders.create_push_constant([1.0, -1]), 16)
-    assert L.refshader_gsplat_render_dispatch(gx, gy, 1, ptrs, sizes, C.cast(push, C.c_void_p), w, h) == 0
-    np.testing.assert_array_equal(bits(tex), bits(want))
+    assert digest(want) == golden("render_fuzz")["rgba"]
 
 
-REF_PLY = "/root/reference/resources/demo.ply"
-
-
-@pytest.mark.skipif(not __import__("os").path.exists(REF_PLY), reason="reference tree not mounted (GPU box)")
-def test_reference_demo_asset_through_the_reference_shaders():
-    """The reference's own demo.ply, 640x480, default camera: every stage of the shaders == the oracle (271 123 splats,
-    M = 428 272, Q10 fires on tile 1198 -- SURVEY Appendix B)."""
-    from godotgaussiansplatting_b200 import camera as cam
-    from godotgaussiansplatting_b200.ply_file import PlyFile
-
-    ply = PlyFile(REF_PLY)
-    s = orc.preprocess_ply(ply.table, 0.0)
-    c = cam.default_camera(aspect=640 / 480)
-    vp = cam.pack_camera_push_constants(c.get_camera_transform(), c.get_camera_projection())
-    from tests.scenes import uniforms_bytes
-    ub = uniforms_bytes([0.0, 0.0, 0.0], 1.0, 640, 480, 10.0)
-    ref, spec = check_scene(s, vp, ub, 640, 480)
-    assert ref.duplicates == 428272 and spec.visible == 226063
-    assert ref.bounds[1198, 1] == 0          # Q10: the last occupied tile never gets its end
+def test_reference_demo_subset_through_the_reference_shaders():
+    """Real data: every 33rd splat of the reference's own demo.ply (tests/golden/demo_subset.npz), 640x480, default camera:
+    every stage of the shaders == the oracle, and Q10 fires on tile 1198 as on the whole asset (SURVEY Appendix B)."""
+    spec, _ = check_scene("demo_subset_640x480", *demo_scene())
+    assert spec.last_tile == 1198
+    assert spec.bounds[1198, 1] == 0          # Q10: the last occupied tile never gets its end
 
 
 def test_boundaries_uninitialised_shared_word():
@@ -270,26 +286,22 @@ def test_boundaries_uninitialised_shared_word():
     spec, _, _ = oracle_frames(splat60, vp, ub, heat)
     T = spec.bounds.shape[0]
     first = int(spec.keys[0] >> 16)
-    for garbage in (0xFFFFFFFF, 0, first + 1, T - 1, first):
-        ref = reference_frame(splat60, vp, ub, w, h, heat, garbage)
-        np.testing.assert_array_equal(ref.bounds, orc.boundaries_uninit(spec.keys, T, garbage), err_msg=f"garbage={garbage:#x}")
+    for garbage in boundaries_garbage_words(spec):
+        got = orc.boundaries_uninit(spec.keys, T, garbage)
+        assert digest(got) == golden(f"boundaries_uninit/{garbage:#x}")["bounds"], f"garbage={garbage:#x}"
         if garbage == first:
-            np.testing.assert_array_equal(ref.bounds, spec.bounds)       # the defined behaviour of orc_boundaries / libgsr
+            np.testing.assert_array_equal(got, spec.bounds)       # the defined behaviour of orc_boundaries / libgsr
         elif garbage != int(spec.keys[1] >> 16):
-            assert ref.bounds[int(spec.keys[1] >> 16), 0] == 1          # a range that starts at 1: instance 0 is dropped
+            assert got[int(spec.keys[1] >> 16), 0] == 1          # a range that starts at 1: instance 0 is dropped
 
 
-@pytest.mark.parametrize("n", [1, 2, 255, 4095, 4096, 4097, 12289, 50000])
+@pytest.mark.parametrize("n", SORT_SIZES)
 def test_sort_shaders_are_a_stable_lsd_sort(n):
-    rng = np.random.default_rng(n)
-    keys = rng.integers(0, 2**32, n, dtype=np.uint64).astype(np.uint32)
-    if n > 1000:
-        keys[: n // 2] = keys[: n // 2] & np.uint32(0xFFFF00FF)       # many ties: stability is observable
-    values = np.arange(n, dtype=np.uint32)
-    k, v = refshaders.sort_pairs(keys, values, cap=n + 17)
+    keys, values = sort_inputs(n)
     order = np.argsort(keys, kind="stable")
-    np.testing.assert_array_equal(k, keys[order])
-    np.testing.assert_array_equal(v, values[order])
+    k, v = keys[order], values[order]
+    ref = golden(f"sort/{n}")
+    assert digest(k) == ref["keys"] and digest(v) == ref["values"]
     ok, ov = orc.sort_pairs(keys, values)
     np.testing.assert_array_equal(k, ok)
     np.testing.assert_array_equal(v, ov)
@@ -301,23 +313,25 @@ def test_sort_shaders_are_a_stable_lsd_sort(n):
 def test_pick_tile():
     """gsplat_render.glsl:105-110 -> tile_splat_pos (rasterizer.gd:162-171)."""
     splat60, vp, ub, w, h, heat = build("default_camera")
-    spec, _, u = oracle_frames(splat60, vp, ub, heat)
-    counts = (spec.bounds[:, 1].astype(np.int64) - spec.bounds[:, 0].astype(np.int64))
-    tile = int(np.argmax(counts))
-    ref = reference_frame(splat60, vp, ub, w, h, heat, int(spec.keys[0] >> 16), target_tile=tile)
+    spec, _, _ = oracle_frames(splat60, vp, ub, heat)
+    tile, counts = pick_target_tile(spec)
     _, _, pick = orc.render(spec.records, spec.values, spec.bounds, w, h, heatmap=heat, target_tile=tile)
-    np.testing.assert_array_equal(bits(ref.pick), bits(pick))
-    assert ref.pick[3] == counts[tile]
+    ref = golden("pick_tile")
+    assert [int(x) for x in bits(pick)] == ref["pick"]
+    assert pick[3] == counts[tile]
 
 
 def test_libm_builtins_stay_inside_tolerance():
     """exp()/pow() are implementation-defined in GLSL: with glibc's expf/powf instead of the spec's polynomials the frame
     stays within the north-star tolerance (a 1-ulp pow() may move a tile rect; allow a vanishing fraction of pixels)."""
     splat60, vp, ub, w, h, heat = build("default_camera")
-    spec, _, _ = oracle_frames(splat60, vp, ub, heat)
-    ref = reference_frame(splat60, vp, ub, w, h, heat, int(spec.keys[0] >> 16), libm=True)
-    assert abs(ref.duplicates - spec.duplicates) <= max(4, spec.duplicates // 10000)
-    bad = (np.abs(ref.rgba - spec.rgba).max(axis=2) > RGBA_TOL).mean()
+    spec, strict, _ = oracle_frames(splat60, vp, ub, heat)
+    assert digest(strict.rgba) == golden("scene/default_camera")["rgba"]
+    ref = golden("libm")
+    assert abs(ref["duplicates"] - spec.duplicates) <= max(4, spec.duplicates // 10000)
+    libm_rgba = strict.rgba.astype(np.float64)
+    libm_rgba[..., :3] += libm_delta() * LIBM_STEP
+    bad = (np.abs(libm_rgba - spec.rgba).max(axis=2) > RGBA_TOL).mean()
     assert bad <= 1e-3, bad
 
 
@@ -328,9 +342,8 @@ def test_cuda_path_against_reference_shaders(name):
     from godotgaussiansplatting_b200 import _lib
     from tests.gsr_direct import Ctx
 
-    n, seed, w, h, frame, time, ms, heat, creation, boost = SCENES[name]
     splat60, vp, ub, w, h, heat = build(name)
-    with Ctx(n, w, h) as c:
+    with Ctx(splat60.shape[0], w, h) as c:
         c.upload(splat60)
         c.keep_unsorted()
         rgba = c.render(vp, ub, heatmap=heat)
@@ -338,14 +351,17 @@ def test_cuda_path_against_reference_shaders(name):
         ukeys = c.copy(_lib.GSR_BUF_KEYS_UNSORTED, t["m"], np.uint32)
         uvals = c.copy(_lib.GSR_BUF_VALUES_UNSORTED, t["m"], np.uint32)
     assert t["m"] > 0
-    ref = reference_frame(splat60, vp, ub, w, h, heat, int(t["keys"][0] >> 16))
-    assert t["m"] == ref.duplicates
-    np.testing.assert_array_equal(ukeys, ref.keys_unsorted)
-    np.testing.assert_array_equal(uvals, ref.values_unsorted)
-    np.testing.assert_array_equal(t["keys"], ref.keys)
-    np.testing.assert_array_equal(t["values"], ref.values)
-    np.testing.assert_array_equal(t["bounds"], ref.bounds)
-    vis = np.unique(ref.values)
+    ref = golden(f"scene/{name}")
+    assert t["m"] == ref["duplicates"]
+    assert digest(ukeys) == ref["keys_unsorted"] and digest(uvals) == ref["values_unsorted"]
+    assert digest(t["keys"]) == ref["keys"] and digest(t["values"]) == ref["values"]
+    assert digest(t["bounds"]) == ref["bounds"]
+    # records and pixels against the oracle's frame, which is the reference shaders' frame (digests checked here too)
+    spec, strict, u = oracle_frames(splat60, vp, ub, heat)
+    assert digest(strict.rgba) == ref["rgba"]
+    pr = orc.project(splat60, vp, u)
+    vis = np.unique(pr.values)
+    assert digest(pr.records[vis]) == ref["records"]
     for f in orc.RECORD_DTYPE.names:
-        np.testing.assert_array_equal(bits(t["records"][f][vis]), bits(ref.records[f][vis]), err_msg=f"record field {f}")
-    assert np.abs(rgba - ref.rgba).max() <= RGBA_TOL
+        np.testing.assert_array_equal(bits(t["records"][f][vis]), bits(pr.records[f][vis]), err_msg=f"record field {f}")
+    assert np.abs(rgba - strict.rgba).max() <= RGBA_TOL
