@@ -19,6 +19,7 @@ GSR_FLAG_REFERENCE_QUIRKS, GSR_FLAG_FIXED_RANGES, GSR_FLAG_FAST_REJECT, GSR_FLAG
 # every symbol include/gsr.h declares (tests/test_abi.py checks the header against this list and the .so)
 EXPORTS = [
     "gsr_create", "gsr_destroy", "gsr_set_stream", "gsr_upload_splats_aos", "gsr_upload_ply_raw", "gsr_resize", "gsr_set_band", "gsr_set_row_interleave", "gsr_band_sync_word", "gsr_band_fixup", "gsr_render",
+    "gsr_set_views", "gsr_render_views", "gsr_render_views_async",
     "gsr_render_async", "gsr_render_async_rgb", "gsr_render_async_fmt", "gsr_output_bytes", "gsr_present_device", "gsr_readback_async", "gsr_peer_export_framebuffers", "gsr_peer_import_framebuffers",
     "gsr_stream_join", "gsr_group_export", "gsr_group_attach", "gsr_group_detach", "gsr_group_set_present", "gsr_readback_rows_async", "gsr_sync", "gsr_framebuffer_device_ptr", "gsr_set_framebuffer_external", "gsr_pick",
     "gsr_get_stats", "gsr_get_frame_history", "gsr_debug_copy", "gsr_debug_enable_trace", "gsr_debug_compositor_config", "gsr_debug_pipeline", "gsr_debug_keep_unsorted", "gsr_sorter_create", "gsr_sorter_destroy",
@@ -43,6 +44,7 @@ GSR_HISTORY_FRAMES = 512
 GSR_OUT_RGBA32F, GSR_OUT_RGB32F, GSR_OUT_RGBA16F, GSR_OUT_RGBA8 = range(4)
 GSR_OUT_SRGB_TO_LINEAR = 0x100
 GSR_GROUP_BLOB_BYTES = 320
+GSR_MAX_VIEWS = 4
 
 
 class GsrFrameRecord(C.Structure):
@@ -81,6 +83,9 @@ def lib():
         L.gsr_band_fixup.argtypes = [vp]
         L.gsr_render.argtypes = [vp, fp, vp, C.c_float, vp]
         L.gsr_render_async.argtypes = [vp, fp, vp, C.c_float, vp]
+        L.gsr_set_views.argtypes = [vp, C.c_int32]
+        L.gsr_render_views.argtypes = [vp, fp, vp, C.c_float, vp]
+        L.gsr_render_views_async.argtypes = [vp, fp, vp, C.c_float, vp, C.c_int32]
         L.gsr_render_async_rgb.argtypes = [vp, fp, vp, C.c_float, vp]
         L.gsr_render_async_fmt.argtypes = [vp, fp, vp, C.c_float, vp, C.c_int32]
         L.gsr_output_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32]

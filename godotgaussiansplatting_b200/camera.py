@@ -33,6 +33,23 @@ def perspective(fovy_degrees: float, aspect: float, z_near: float, z_far: float)
     return m.reshape(16)
 
 
+def frustum(left: float, right: float, bottom: float, top: float, z_near: float, z_far: float) -> np.ndarray:
+    """Godot `Projection.create_frustum` (Projection::set_frustum): an off-axis perspective with the near-plane window
+    [left, right] x [bottom, top], as OpenXR hands each eye (XRInterface.get_projection_for_view).  16 float32, column-major.
+    The off-centre terms sit in column z (m[2][0], m[2][1]): they shift a splat's image position by a constant per depth, and the EWA
+    Jacobian of the projection reads only m[0][0] and m[1][1]."""
+    l, r, b, t, n, f = (F(v) for v in (left, right, bottom, top, z_near, z_far))
+    m = np.zeros((4, 4), dtype=np.float32)  # m[c][r]
+    m[0][0] = F(2.0) * n / (r - l)
+    m[1][1] = F(2.0) * n / (t - b)
+    m[2][0] = (r + l) / (r - l)
+    m[2][1] = (t + b) / (t - b)
+    m[2][2] = -(f + n) / (f - n)
+    m[2][3] = F(-1.0)
+    m[3][2] = -(F(2.0) * f * n) / (f - n)
+    return m.reshape(16)
+
+
 def transform_to_projection(basis_cols: np.ndarray, origin: np.ndarray) -> np.ndarray:
     """Godot Projection(Transform3D): columns (x,0),(y,0),(z,0),(origin,1)."""
     m = np.zeros((4, 4), dtype=np.float32)
@@ -118,6 +135,19 @@ def orbit_camera(frame: int, center=(0.0, 0.0, 2.5), radius: float = 2.5, pitch_
     cam.aspect = aspect
     cam.look_at_from_position(pos, cw)
     return cam
+
+
+def stereo_pair(camera: Camera3D, ipd: float = 0.063) -> tuple[Camera3D, Camera3D]:
+    """(left, right) eyes of `camera`: the same orientation and projection, positions offset by -ipd/2 and +ipd/2 along the
+    camera's right axis (basis column x) -- what an XR runtime's per-view transforms are for a head pose."""
+    eyes = []
+    for sign in (-0.5, 0.5):
+        e = Camera3D(fov=camera.fov, near=camera.near, far=camera.far)
+        e.aspect = camera.aspect
+        e.basis = camera.basis.copy()
+        e.global_position = (camera.global_position.astype(np.float64) + sign * float(ipd) * camera.basis[0].astype(np.float64)).astype(np.float32)
+        eyes.append(e)
+    return eyes[0], eyes[1]
 
 
 def default_camera(aspect: float = 16.0 / 9.0, fov: float = 75.0) -> Camera3D:

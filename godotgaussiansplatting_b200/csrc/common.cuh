@@ -157,6 +157,16 @@ struct ProjectionArgs {
 };
 int launch_projection(const ProjectionArgs &a, cudaStream_t stream);
 
+// Multiview frame (gsr_set_views): K cameras of one splat cloud in one projection.  view[v] carries camera v's matrices, uniform block
+// and per-frame constants and its own record table; every other field is the same in all K entries (keys, values, capacity, look-back,
+// frame state, splat planes).  View v's pairs carry the tile ids [v*T, (v+1)*T), so one sort orders all views.
+struct ViewsArgs {
+    ProjectionArgs view[GSR_MAX_VIEWS];
+    int32_t num_views;
+    uint32_t tiles_per_view;  // T
+};
+int launch_projection_views(const ViewsArgs &a, cudaStream_t stream);
+
 // ---------------------------------------------------------------------------------------------
 // multi-GPU shard group (group.cu, gsr_group_attach): flag words + receive segments + record tables in every rank's arena
 // ---------------------------------------------------------------------------------------------
@@ -219,6 +229,10 @@ uint32_t projection_num_blocks(uint32_t num_splats);
 // (local last tile -> *sync_word = tile + 1; the frame-global quirk is applied later by launch_band_fixup).
 int launch_tile_ranges(const uint32_t *sorted_keys, const FrameState *frame, uint2 *bounds, uint32_t num_tiles,
                        int quirks, int sharded, int32_t *sync_word, int grid, cudaStream_t stream);
+// Multiview frame: the same ranges per view over the concatenated tile ids (view = tile / tiles_per_view).  Each view's last key gets
+// the single-view tail rule (Q10 with T-1 = the view's last tile); the plain end of a view's last tile is never written.
+int launch_tile_ranges_views(const uint32_t *sorted_keys, const FrameState *frame, uint2 *bounds, uint32_t tiles_per_view, int quirks, int grid,
+                             cudaStream_t stream);
 int launch_band_fixup(const int32_t *global_last_plus1, float4 *out, int32_t width, int32_t height, int32_t tiles_x, int32_t num_tiles_total,
                       int32_t band_y0, int32_t band_y1, int32_t row_mod, int32_t row_rem, cudaStream_t stream);
 
@@ -244,6 +258,11 @@ struct CompositeArgs {
     ulonglong4 *trace;       // optional schedule trace (debug): {tile<<32|smid, t0_ns, t1_ns, consumed<<32|list_chunks<<1|1}
     uint32_t *trace_count;
     uint32_t trace_cap;
+    // multiview frame (zero = one view): tile id t renders tile t % tiles_per_view of view t / tiles_per_view, from record table
+    // `records + view * record_stride` (float4s) into layer `out + view * layer_stride` (pixels)
+    int32_t tiles_per_view;
+    uint64_t layer_stride;
+    uint64_t record_stride;
 };
 int launch_composite(const CompositeArgs &a, cudaStream_t stream);
 int composite_max_ctas_per_sm(int *out);

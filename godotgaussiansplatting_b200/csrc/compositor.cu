@@ -220,8 +220,9 @@ __device__ __forceinline__ void phase_b(const float4 B[GU], const float *s_c, in
 #endif
 
 // Persistent CTAs.  Ticket k of the launch renders owned tile order[k] (longest chains first) or k itself; every tile is blended
-// from its first chunk to its stop by the CTA that took it.
-template <bool CONTRACT>
+// from its first chunk to its stop by the CTA that took it.  MULTI: a multiview frame (CompositeArgs::tiles_per_view), whose tile id
+// selects the view's record table and frame layer; the blend itself is the same code.
+template <bool CONTRACT, bool MULTI = false>
 __global__ void __launch_bounds__(THREADS, GSR_COMP_MIN_BLOCKS) composite_kernel(const __grid_constant__ CompositeArgs p) {
     __shared__ float4 s_a[CHUNK];
     __shared__ float4 s_b[CHUNK];
@@ -249,8 +250,17 @@ __global__ void __launch_bounds__(THREADS, GSR_COMP_MIN_BLOCKS) composite_kernel
         if (local_tile == 0xFFFFFFFFu) break;
         // owned tiles: rows tile_begin/tiles_x + k*row_step, all columns (row_step == 1: one contiguous band)
         const uint32_t tile_id = (uint32_t)p.tile_begin + (local_tile / (uint32_t)p.tiles_x) * (uint32_t)(p.row_step * p.tiles_x) + local_tile % (uint32_t)p.tiles_x;
+        const float4 *records = p.records;
+        float4 *out = p.out;
+        uint32_t view_tile = tile_id;
+        if (MULTI) {
+            const uint32_t view = tile_id / (uint32_t)p.tiles_per_view;
+            view_tile = tile_id - view * (uint32_t)p.tiles_per_view;
+            records += (uint64_t)view * p.record_stride;
+            out += (uint64_t)view * p.layer_stride;
+        }
 
-        const uint32_t tx = tile_id % (uint32_t)p.tiles_x, ty = tile_id / (uint32_t)p.tiles_x;
+        const uint32_t tx = view_tile % (uint32_t)p.tiles_x, ty = view_tile / (uint32_t)p.tiles_x;
         const int px0 = (int)(tx * TILE + 2u * (tid & 7u)), py = (int)(ty * TILE + (tid >> 3));
         const u64 npx2 = pk(-(float)px0, -(float)(px0 + 1));  // ox = image_pos.x - pixel.x  ==  image_pos.x + (-pixel.x)
         const float fpy = (float)py;
@@ -265,8 +275,8 @@ __global__ void __launch_bounds__(THREADS, GSR_COMP_MIN_BLOCKS) composite_kernel
 
         Staged n0 = null_splat(), n1 = null_splat();
         if (num_iterations > 0) {
-            if ((int)tid < num_splats) n0 = gather(p.records, p.values, bounds.x + tid);
-            if ((int)tid + THREADS < num_splats) n1 = gather(p.records, p.values, bounds.x + tid + THREADS);
+            if ((int)tid < num_splats) n0 = gather(records, p.values, bounds.x + tid);
+            if ((int)tid + THREADS < num_splats) n1 = gather(records, p.values, bounds.x + tid + THREADS);
         }
 
         int consumed = 0;  // chunks blended before the stop rule fired (next frame's scheduling hint)
@@ -282,8 +292,8 @@ __global__ void __launch_bounds__(THREADS, GSR_COMP_MIN_BLOCKS) composite_kernel
             n0 = null_splat(); n1 = null_splat();
             if (i + 1 < num_iterations) {
                 const int nb = sort_offset + CHUNK;
-                if (nb + (int)tid < num_splats) n0 = gather(p.records, p.values, bounds.x + (uint32_t)nb + tid);
-                if (nb + (int)tid + THREADS < num_splats) n1 = gather(p.records, p.values, bounds.x + (uint32_t)nb + tid + THREADS);
+                if (nb + (int)tid < num_splats) n0 = gather(records, p.values, bounds.x + (uint32_t)nb + tid);
+                if (nb + (int)tid + THREADS < num_splats) n1 = gather(records, p.values, bounds.x + (uint32_t)nb + tid + THREADS);
             }
 
             // :79-91, GU splats per iteration; `chunk` rounded up to GU reads null splats (opacity 0 => exact no-op).  Software-pipelined:
@@ -324,7 +334,7 @@ __global__ void __launch_bounds__(THREADS, GSR_COMP_MIN_BLOCKS) composite_kernel
         const float hx = (float)num_splats * 5e-4f;
         const float h0 = 0.0f * (1.0f - hx) + 1.0f * hx, h1 = 0.0f * (1.0f - hx) + 0.2f * hx, h2c = 1.0f * (1.0f - hx) + 0.2f * hx;
         if (py < p.height) {
-            float4 *row = p.out + (uint64_t)py * (uint64_t)p.width;
+            float4 *row = out + (uint64_t)py * (uint64_t)p.width;
             const float k0 = 1.0f - t0, k1 = 1.0f - t1;
             if (px0 < p.width)
                 row[px0] = make_float4(r0 + h0 * k0 * p.heatmap_factor, g0 + h1 * k0 * p.heatmap_factor, b0 + h2c * k0 * p.heatmap_factor, 1.0f);
@@ -335,7 +345,7 @@ __global__ void __launch_bounds__(THREADS, GSR_COMP_MIN_BLOCKS) composite_kernel
         // index 32*s = pixel (0, 2*s) of the tile = first pixel of thread 16*s here
         if ((tid & 15u) == 0u && tile_id == p.target_tile_id && t0 != 1.0f) {
             const uint32_t v = p.values[bounds.x + (bounds.y - bounds.x) / 10u];
-            const float4 q0 = p.records[(uint64_t)v * 3u + 0], q1 = p.records[(uint64_t)v * 3u + 1];
+            const float4 q0 = records[(uint64_t)v * 3u + 0], q1 = records[(uint64_t)v * 3u + 1];
             *p.pick = make_float4(q0.z, q0.w, q1.w, (float)num_splats);
         }
         if (tid == 0) {
@@ -356,15 +366,17 @@ __global__ void __launch_bounds__(THREADS, GSR_COMP_MIN_BLOCKS) composite_kernel
 #ifndef GSR_CPU_EMU
 int preload_composite_kernels() {
     cudaFuncAttributes fa;
-    GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, composite_kernel<true>));
-    GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, composite_kernel<false>));
+    GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, composite_kernel<true, false>));
+    GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, composite_kernel<false, false>));
+    GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, composite_kernel<true, true>));
+    GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, composite_kernel<false, true>));
     return GSR_OK;
 }
 
 int composite_max_ctas_per_sm(int *out) {
     int a = 0, b = 0;
-    GSR_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, composite_kernel<true>, THREADS, 0));
-    GSR_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, composite_kernel<false>, THREADS, 0));
+    GSR_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, composite_kernel<true, false>, THREADS, 0));
+    GSR_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, composite_kernel<false, false>, THREADS, 0));
     *out = a < b ? a : b;
     if (*out < 1) *out = 1;
     return GSR_OK;
@@ -374,8 +386,13 @@ int launch_composite(const CompositeArgs &a, cudaStream_t stream) {
     if (a.num_tiles <= 0) return GSR_OK;
     const int per_sm = a.ctas_per_sm > 0 ? a.ctas_per_sm : 1;
     const int grid = a.num_tiles < a.sm_count * per_sm ? a.num_tiles : a.sm_count * per_sm;
-    if (a.contract) composite_kernel<true><<<grid, THREADS, 0, stream>>>(a);
-    else composite_kernel<false><<<grid, THREADS, 0, stream>>>(a);
+    if (a.tiles_per_view > 0) {
+        if (a.contract) composite_kernel<true, true><<<grid, THREADS, 0, stream>>>(a);
+        else composite_kernel<false, true><<<grid, THREADS, 0, stream>>>(a);
+    } else {
+        if (a.contract) composite_kernel<true, false><<<grid, THREADS, 0, stream>>>(a);
+        else composite_kernel<false, false><<<grid, THREADS, 0, stream>>>(a);
+    }
     GSR_CUDA_TRY(cudaGetLastError());
     return GSR_OK;
 }

@@ -110,6 +110,9 @@ struct gsr_ctx {
     bool ev_valid = false;
     uint32_t last_launches = 0;
     int sm_count = 0;
+    // multiview frame (gsr_set_views): K layers of W*H pixels, K*T tile bounds, K record tables of 3 * max_splats float4 per table
+    int num_views = 1;
+    uint64_t cap_factor = 10;    // gsr_config.dup_capacity_factor: the initial capacity is num_views * factor * max_splats
 };
 
 struct gsr_sorter {
@@ -158,6 +161,13 @@ void group_detach(gsr_ctx *c) {
 }
 
 float4 *framebuffer(gsr_ctx *c) { return c->fb_ext ? c->fb_ext : (c->fb_last ? c->fb_last : c->fb); }
+// pixels of a frame (all layers) and tiles of a frame (all views)
+size_t frame_pixels(const gsr_ctx *c) { return (size_t)c->width * c->height * (size_t)c->num_views; }
+size_t frame_tiles(const gsr_ctx *c) { return (size_t)c->tiles_x * c->tiles_y * (size_t)c->num_views; }
+int refuse_multiview(const char *what) {
+    set_last_error("%s: unavailable in a multiview context (gsr_set_views > 1)", what);
+    return GSR_ERR_STATE;
+}
 
 void free_ctx(gsr_ctx *c) {
     if (!c) return;
@@ -226,6 +236,7 @@ GSR_API int gsr_create(const gsr_config *cfg, gsr_ctx **out) {
     if (!(c->flags & (GSR_FLAG_REFERENCE_QUIRKS | GSR_FLAG_FIXED_RANGES))) c->flags |= GSR_FLAG_REFERENCE_QUIRKS;
     c->max_splats = cfg->max_splats;
     const uint64_t factor = cfg->dup_capacity_factor ? cfg->dup_capacity_factor : 10;  // rasterizer.gd:79
+    c->cap_factor = factor;
     c->capacity_max = (1ull << 30) - 1;  // look-back words carry 30-bit counts
     c->capacity = c->max_splats * factor;
     if (c->capacity > c->capacity_max) c->capacity = c->capacity_max;
@@ -369,10 +380,11 @@ GSR_API int gsr_upload_ply_raw(gsr_ctx *c, const float *ply, uint32_t nprops, ui
 GSR_API int gsr_resize(gsr_ctx *c, int32_t width, int32_t height) {
     if (!c || width < 1 || height < 1) { set_last_error("gsr_resize: bad size %dx%d", width, height); return GSR_ERR_INVALID; }
     const int tx = (width + TILE - 1) / TILE, ty = (height + TILE - 1) / TILE;
-    if ((int64_t)tx * ty > 65536) {  // tile id must fit the 16 key bits above the depth code (gsplat_projection.glsl:222)
-        set_last_error("gsr_resize: %d tiles exceed the 16-bit tile id of the sort key", tx * ty);
+    if ((int64_t)tx * ty * c->num_views > 65536) {  // tile id must fit the 16 key bits above the depth code (gsplat_projection.glsl:222)
+        set_last_error("gsr_resize: %d views x %d tiles exceed the 16-bit tile id of the sort key", c->num_views, tx * ty);
         return GSR_ERR_INVALID;
     }
+    const size_t K = (size_t)c->num_views;
     int rc = use_device(c->device);
     if (rc) return rc;
     GSR_CUDA_TRY(cudaStreamSynchronize(c->front_stream));
@@ -392,16 +404,16 @@ GSR_API int gsr_resize(gsr_ctx *c, int32_t width, int32_t height) {
     if (c->peer_opened) { cudaIpcCloseMemHandle(c->peer_fb[0]); cudaIpcCloseMemHandle(c->peer_fb[1]); c->peer_opened = false; }
     c->peer_mode = false; c->peer_fb[0] = c->peer_fb[1] = nullptr; c->peer_counter = 0; c->async_counter = 0;
     group_detach(c);   // same for a shard group: every rank resizes, exports and attaches again
-    GSR_CUDA_TRY(cudaMalloc((void **)&c->bounds, sizeof(uint2) * (size_t)tx * ty));
-    GSR_CUDA_TRY(cudaMalloc((void **)&c->comp_order, sizeof(uint32_t) * (size_t)tx * ty));
-    GSR_CUDA_TRY(cudaMalloc((void **)&c->comp_hint, sizeof(uint32_t) * (size_t)tx * ty));
-    GSR_CUDA_TRY(cudaMemsetAsync(c->comp_hint, 0, sizeof(uint32_t) * (size_t)tx * ty, c->stream));
+    GSR_CUDA_TRY(cudaMalloc((void **)&c->bounds, sizeof(uint2) * (size_t)tx * ty * K));
+    GSR_CUDA_TRY(cudaMalloc((void **)&c->comp_order, sizeof(uint32_t) * (size_t)tx * ty * K));
+    GSR_CUDA_TRY(cudaMalloc((void **)&c->comp_hint, sizeof(uint32_t) * (size_t)tx * ty * K));
+    GSR_CUDA_TRY(cudaMemsetAsync(c->comp_hint, 0, sizeof(uint32_t) * (size_t)tx * ty * K, c->stream));
     c->comp_hint_key = 0;
     if (!c->pick_frame) GSR_CUDA_TRY(cudaMalloc((void **)&c->pick_frame, sizeof(FrameState)));
-    GSR_CUDA_TRY(cudaMalloc((void **)&c->fb, sizeof(float4) * (size_t)width * height));
-    GSR_CUDA_TRY(cudaMalloc((void **)&c->fb2, sizeof(float4) * (size_t)width * height));
-    GSR_CUDA_TRY(cudaMemsetAsync(c->fb, 0, sizeof(float4) * (size_t)width * height, c->stream));
-    GSR_CUDA_TRY(cudaMemsetAsync(c->fb2, 0, sizeof(float4) * (size_t)width * height, c->stream));
+    GSR_CUDA_TRY(cudaMalloc((void **)&c->fb, sizeof(float4) * (size_t)width * height * K));
+    GSR_CUDA_TRY(cudaMalloc((void **)&c->fb2, sizeof(float4) * (size_t)width * height * K));
+    GSR_CUDA_TRY(cudaMemsetAsync(c->fb, 0, sizeof(float4) * (size_t)width * height * K, c->stream));
+    GSR_CUDA_TRY(cudaMemsetAsync(c->fb2, 0, sizeof(float4) * (size_t)width * height * K, c->stream));
     c->width = width; c->height = height; c->tiles_x = tx; c->tiles_y = ty;
     if (!c->band_set) { c->band_y0 = 0; c->band_y1 = ty; }
     if (c->band_y1 > ty) c->band_y1 = ty;
@@ -411,6 +423,7 @@ GSR_API int gsr_resize(gsr_ctx *c, int32_t width, int32_t height) {
 
 GSR_API int gsr_set_row_interleave(gsr_ctx *c, int32_t row_rem, int32_t row_mod) {
     if (!c || row_mod < 1 || row_rem < 0 || row_rem >= row_mod) { set_last_error("gsr_set_row_interleave: need 0 <= rem < mod"); return GSR_ERR_INVALID; }
+    if (c->num_views > 1 && row_mod > 1) return refuse_multiview("gsr_set_row_interleave");
     c->row_mod = row_mod; c->row_rem = row_rem;
     return GSR_OK;
 }
@@ -430,9 +443,45 @@ GSR_API int gsr_band_fixup(gsr_ctx *c) {
 GSR_API int gsr_set_band(gsr_ctx *c, int32_t row_begin, int32_t row_end) {
     if (!c || c->tiles_y == 0) { set_last_error("gsr_set_band before gsr_resize"); return GSR_ERR_STATE; }
     if (row_begin < 0 || row_end > c->tiles_y || row_begin > row_end) { set_last_error("band [%d,%d) outside [0,%d]", row_begin, row_end, c->tiles_y); return GSR_ERR_INVALID; }
+    if (c->num_views > 1 && !(row_begin == 0 && row_end == c->tiles_y)) return refuse_multiview("gsr_set_band");
     c->band_y0 = row_begin; c->band_y1 = row_end;
     c->band_set = !(row_begin == 0 && row_end == c->tiles_y);
     return GSR_OK;
+}
+
+static int grow_capacity(gsr_ctx *c, uint64_t want);
+
+GSR_API int gsr_set_views(gsr_ctx *c, int32_t num_views) {
+    if (!c || num_views < 1 || num_views > GSR_MAX_VIEWS) { set_last_error("gsr_set_views: need a context and 1 <= views <= %d", GSR_MAX_VIEWS); return GSR_ERR_INVALID; }
+    if ((int64_t)c->tiles_x * c->tiles_y * num_views > 65536) {
+        set_last_error("gsr_set_views: %d views x %d tiles exceed the 16-bit tile id of the sort key", num_views, c->tiles_x * c->tiles_y);
+        return GSR_ERR_INVALID;
+    }
+    if (num_views > 1 && (c->grp.world > 1 || c->peer_mode || c->band_set || !(c->band_y0 == 0 && c->band_y1 == c->tiles_y) || c->row_mod > 1 ||
+                          c->overlap > 0)) {
+        set_last_error("gsr_set_views: multiview needs a single-GPU full-frame context (no shard group, peer frames, band, row interleave or overlap)");
+        return GSR_ERR_STATE;
+    }
+    if (num_views == c->num_views) return GSR_OK;
+    int rc = use_device(c->device);
+    if (rc) return rc;
+    GSR_CUDA_TRY(cudaStreamSynchronize(c->front_stream));
+    GSR_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    GSR_CUDA_TRY(cudaStreamSynchronize(c->copy_stream));
+    // one record table per view, in each of the two alternating sets
+    cudaFree(c->records); cudaFree(c->records2);
+    c->records = c->records2 = c->records_cur = nullptr;
+    const size_t rec_bytes = sizeof(float4) * 3ull * c->max_splats * (size_t)num_views;
+    GSR_CUDA_TRY(cudaMalloc((void **)&c->records, rec_bytes));
+    GSR_CUDA_TRY(cudaMalloc((void **)&c->records2, rec_bytes));
+    GSR_CUDA_TRY(cudaMemsetAsync(c->records, 0, rec_bytes, c->stream));
+    GSR_CUDA_TRY(cudaMemsetAsync(c->records2, 0, rec_bytes, c->stream));
+    c->records_cur = c->records;
+    c->num_views = num_views;
+    // K-layer frames, K*T bounds / compositor order / hints (the hints are dropped)
+    if (c->width > 0 && (rc = gsr_resize(c, c->width, c->height))) return rc;
+    // every view brings its own duplicates: start from K x factor x N, like K single-view contexts (grows on demand as before)
+    return grow_capacity(c, (uint64_t)num_views * c->cap_factor * c->max_splats);
 }
 
 // Per-frame constants of the projection: project_covariance's focal / limit terms and the norm bound of the conservative reject.
@@ -541,11 +590,20 @@ static int render_enqueue(gsr_ctx *c, const float *view_proj, const void *unifor
                           const GroupFrame *gf = nullptr) {
     if (!c || !view_proj || !uniforms32) return GSR_ERR_INVALID;
     if (c->width == 0) { set_last_error("gsr_render before gsr_resize"); return GSR_ERR_STATE; }
+    const int K = c->num_views;   // view_proj / uniforms32: K push constants / uniform blocks
     Uniforms u;
     memcpy(&u, uniforms32, sizeof u);
     if (u.dims[0] != c->width || u.dims[1] != c->height) {
         set_last_error("uniform dims %dx%d differ from gsr_resize %dx%d", u.dims[0], u.dims[1], c->width, c->height);
         return GSR_ERR_INVALID;
+    }
+    for (int v = 1; v < K; ++v) {   // the fused projection shares the time factors, scaled covariance and opacity between views
+        Uniforms uv;
+        memcpy(&uv, static_cast<const char *>(uniforms32) + sizeof(Uniforms) * v, sizeof uv);
+        if (memcmp(&uv.model_scale, &u.model_scale, sizeof u.model_scale) || memcmp(uv.dims, u.dims, sizeof u.dims) || memcmp(&uv.time, &u.time, sizeof u.time)) {
+            set_last_error("uniform block of view %d differs from view 0 in model_scale, width, height or time", v);
+            return GSR_ERR_INVALID;
+        }
     }
     int rc = use_device(c->device);
     if (rc) return rc;
@@ -567,7 +625,7 @@ static int render_enqueue(gsr_ctx *c, const float *view_proj, const void *unifor
     uint32_t *keys_in = c->keys + (size_t)half * c->cap_stride, *vals_in = c->vals + (size_t)half * c->cap_stride;
     uint32_t *keys_alt = c->keys + 2ull * c->cap_stride, *vals_alt = c->vals + 2ull * c->cap_stride;
     float4 *records = half ? c->records2 : c->records;
-    const uint32_t n_tiles = (uint32_t)(c->tiles_x * c->tiles_y);
+    const uint32_t n_tiles = (uint32_t)frame_tiles(c);
 
     // ---- front: rasterizer.gd:127-128 (clear M = this frame's history slot + the scan links), then the projection ----
     if (overlap && c->front_gate) GSR_CUDA_TRY(cudaStreamWaitEvent(fs, c->front_gate, 0));
@@ -628,6 +686,20 @@ static int render_enqueue(gsr_ctx *c, const float *view_proj, const void *unifor
         sp.lookback = c->lookback;
         if ((rc = launch_projection_scatter(pa, sp, fs))) return rc;
         launches += 1;
+    } else if (K > 1) {
+        ViewsArgs va;
+        memset(&va, 0, sizeof va);
+        va.num_views = K; va.tiles_per_view = (uint32_t)(c->tiles_x * c->tiles_y);
+        for (int v = 0; v < K; ++v) {
+            ProjectionArgs &pv = va.view[v];
+            pv = pa;
+            memcpy(pv.vp, view_proj + 32 * v, sizeof pv.vp);
+            memcpy(&pv.u, static_cast<const char *>(uniforms32) + sizeof(Uniforms) * v, sizeof pv.u);
+            frame_constants(view_proj + 32 * v, pv.u, pv);
+            pv.records = records + 3ull * c->max_splats * (uint64_t)v;
+        }
+        if ((rc = launch_projection_views(va, fs))) return rc;
+        launches += pa.num_splats ? 1 : 0;
     } else {
         if ((rc = launch_projection(pa, fs))) return rc;
         launches += pa.num_splats ? 1 : 0;
@@ -666,7 +738,9 @@ static int render_enqueue(gsr_ctx *c, const float *view_proj, const void *unifor
     const int sharded = fast ? 2 : ((!(c->band_y0 == 0 && c->band_y1 == c->tiles_y) || c->row_mod > 1) ? 1 : 0);
     if (fast) GSR_CUDA_TRY(cudaMemsetAsync(c->sync_word, 0, sizeof(int32_t), s));
     const int quirks = (c->flags & GSR_FLAG_FIXED_RANGES) ? 0 : 1;
-    if ((rc = launch_tile_ranges(keys_in, c->frame, c->bounds, n_tiles, quirks, sharded, fast ? c->sync_word : nullptr, c->sm_count * 8, s))) return rc;
+    if (K > 1) rc = launch_tile_ranges_views(keys_in, c->frame, c->bounds, (uint32_t)(c->tiles_x * c->tiles_y), quirks, c->sm_count * 8, s);
+    else rc = launch_tile_ranges(keys_in, c->frame, c->bounds, n_tiles, quirks, sharded, fast ? c->sync_word : nullptr, c->sm_count * 8, s);
+    if (rc) return rc;
     launches += 1;
     GSR_CUDA_TRY(cudaEventRecord(ev[5], s));  // 'Boundaries'
     c->front_gate = ev[5];   // the next frame's front part may start here, beside this frame's compositor
@@ -686,8 +760,11 @@ static int render_enqueue(gsr_ctx *c, const float *view_proj, const void *unifor
         int nrows = first < c->band_y1 ? (c->band_y1 - 1 - first) / c->row_mod + 1 : 0;
         ca.tile_begin = first * c->tiles_x;
         ca.row_step = c->row_mod;
-        ca.num_tiles = nrows * c->tiles_x;
+        ca.num_tiles = nrows * c->tiles_x * K;   // K > 1: full frame (no band, no rows), so the owned tiles are all K*T
     }
+    ca.tiles_per_view = K > 1 ? c->tiles_x * c->tiles_y : 0;
+    ca.layer_stride = (uint64_t)c->width * c->height;
+    ca.record_stride = 3ull * c->max_splats;
     ca.heatmap_factor = heatmap_factor;
     ca.target_tile_id = 0xFFFFFFFFu;  // rasterizer.gd:158
     ca.pick = c->pick;
@@ -697,7 +774,7 @@ static int render_enqueue(gsr_ctx *c, const float *view_proj, const void *unifor
     ca.contract = (c->flags & GSR_FLAG_UNCONTRACTED_BLEND) ? 0 : 1;
     {   // the hints describe the owned-tile indexing of the frame that wrote them: drop them when the ownership changes
         const uint64_t key = ((uint64_t)(uint32_t)ca.tile_begin << 32) ^ ((uint64_t)(uint32_t)ca.row_step << 24) ^ (uint64_t)(uint32_t)ca.num_tiles;
-        if (key != c->comp_hint_key) { GSR_CUDA_TRY(cudaMemsetAsync(c->comp_hint, 0, sizeof(uint32_t) * (size_t)c->tiles_x * c->tiles_y, s)); c->comp_hint_key = key; }
+        if (key != c->comp_hint_key) { GSR_CUDA_TRY(cudaMemsetAsync(c->comp_hint, 0, sizeof(uint32_t) * frame_tiles(c), s)); c->comp_hint_key = key; }
     }
     if (c->comp_order_mode && ca.num_tiles > 0) {   // longest chains first: the long sequential chains start at once instead of in the tail
         if ((rc = launch_tile_order(c->bounds, ca.tile_begin, ca.row_step, ca.tiles_x, ca.num_tiles, c->comp_hint, c->comp_order, c->frame,
@@ -729,7 +806,7 @@ static int render_enqueue(gsr_ctx *c, const float *view_proj, const void *unifor
     return GSR_OK;
 }
 
-GSR_API int gsr_render(gsr_ctx *c, const float view_proj[32], const void *uniforms32, float heatmap_factor, float *out_host) {
+static int render_sync_impl(gsr_ctx *c, const float *view_proj, const void *uniforms32, float heatmap_factor, float *out_host) {
     if (c && c->grp.world > 1) { set_last_error("gsr_render: a context attached to a group renders with gsr_render_async (all ranks, same frame)"); return GSR_ERR_STATE; }
     int rc = render_enqueue(c, view_proj, uniforms32, heatmap_factor);
     if (rc) return rc;
@@ -744,14 +821,23 @@ GSR_API int gsr_render(gsr_ctx *c, const float view_proj[32], const void *unifor
             if ((rc = grow_capacity(c, fs.dup_total + fs.dup_total / 4ull + 1024ull))) return rc;
             if ((rc = render_enqueue(c, view_proj, uniforms32, heatmap_factor))) return rc;
         }
-        GSR_CUDA_TRY(cudaMemcpyAsync(out_host, framebuffer(c), sizeof(float4) * (size_t)c->width * c->height, cudaMemcpyDeviceToHost, c->stream));
+        GSR_CUDA_TRY(cudaMemcpyAsync(out_host, framebuffer(c), sizeof(float4) * frame_pixels(c), cudaMemcpyDeviceToHost, c->stream));
         GSR_CUDA_TRY(cudaStreamSynchronize(c->stream));
     }
     return GSR_OK;
 }
 
+GSR_API int gsr_render(gsr_ctx *c, const float view_proj[32], const void *uniforms32, float heatmap_factor, float *out_host) {
+    if (c && c->num_views > 1) return refuse_multiview("gsr_render (use gsr_render_views)");
+    return render_sync_impl(c, view_proj, uniforms32, heatmap_factor, out_host);
+}
+
+GSR_API int gsr_render_views(gsr_ctx *c, const float *view_proj, const void *uniforms, float heatmap_factor, float *out_host) {
+    return render_sync_impl(c, view_proj, uniforms, heatmap_factor, out_host);
+}
+
 static int readback_enqueue(gsr_ctx *c, float4 *frame, int slot, void *pinned_host, int format, uint32_t group_seq = 0) {
-    const size_t pixels = (size_t)c->width * c->height;
+    const size_t pixels = frame_pixels(c);
     const size_t bpp = present_bytes_per_pixel(format);
     if (!bpp) { set_last_error("unknown output format 0x%x", format); return GSR_ERR_INVALID; }
     int rc;
@@ -808,7 +894,7 @@ static int render_async_impl(gsr_ctx *c, const float *view_proj, const void *uni
         int rc = render_enqueue(c, view_proj, uniforms32, heatmap_factor);
         if (rc) return rc;
         if (pinned_host)
-            GSR_CUDA_TRY(cudaMemcpyAsync(pinned_host, framebuffer(c), sizeof(float4) * (size_t)c->width * c->height, cudaMemcpyDeviceToHost, c->stream));
+            GSR_CUDA_TRY(cudaMemcpyAsync(pinned_host, framebuffer(c), sizeof(float4) * frame_pixels(c), cudaMemcpyDeviceToHost, c->stream));
         return GSR_OK;
     }
     // Pipelined read-back: frames alternate between two device framebuffers; the D2H copy of frame i runs on the
@@ -825,16 +911,24 @@ static int render_async_impl(gsr_ctx *c, const float *view_proj, const void *uni
 }
 
 GSR_API int gsr_render_async(gsr_ctx *c, const float view_proj[32], const void *uniforms32, float heatmap_factor, float *pinned_host) {
+    if (c && c->num_views > 1) return refuse_multiview("gsr_render_async (use gsr_render_views_async)");
     return render_async_impl(c, view_proj, uniforms32, heatmap_factor, pinned_host, GSR_OUT_RGBA32F);
 }
 
 GSR_API int gsr_render_async_rgb(gsr_ctx *c, const float view_proj[32], const void *uniforms32, float heatmap_factor, float *pinned_host_rgb) {
+    if (c && c->num_views > 1) return refuse_multiview("gsr_render_async_rgb (use gsr_render_views_async)");
     return render_async_impl(c, view_proj, uniforms32, heatmap_factor, pinned_host_rgb, GSR_OUT_RGB32F);
 }
 
 GSR_API int gsr_render_async_fmt(gsr_ctx *c, const float view_proj[32], const void *uniforms32, float heatmap_factor, void *pinned_host, int32_t format) {
+    if (c && c->num_views > 1) return refuse_multiview("gsr_render_async_fmt (use gsr_render_views_async)");
     if (!present_bytes_per_pixel(format)) { set_last_error("unknown output format 0x%x", format); return GSR_ERR_INVALID; }
     return render_async_impl(c, view_proj, uniforms32, heatmap_factor, pinned_host, format);
+}
+
+GSR_API int gsr_render_views_async(gsr_ctx *c, const float *view_proj, const void *uniforms, float heatmap_factor, void *pinned_host, int32_t format) {
+    if (!present_bytes_per_pixel(format)) { set_last_error("unknown output format 0x%x", format); return GSR_ERR_INVALID; }
+    return render_async_impl(c, view_proj, uniforms, heatmap_factor, pinned_host, format);
 }
 
 GSR_API size_t gsr_output_bytes(int32_t format, int32_t width, int32_t height) {
@@ -853,7 +947,7 @@ GSR_API int gsr_present_device(gsr_ctx *c, void *dst_device, int32_t format) {
         if (c->grp.rank != 0) { set_last_error("gsr_present_device: only rank 0 of a group presents the frame"); return GSR_ERR_STATE; }
         if ((rc = launch_group_wait_done(c->grp.flags[0], c->grp.world, c->grp.seq, c->stream))) return rc;
     }
-    return launch_present(framebuffer(c), dst_device, (uint64_t)c->width * c->height, format, c->stream);
+    return launch_present(framebuffer(c), dst_device, (uint64_t)frame_pixels(c), format, c->stream);
 }
 
 GSR_API int gsr_readback_async(gsr_ctx *c, void *pinned_host, int32_t format) {
@@ -908,6 +1002,7 @@ GSR_API int gsr_readback_rows_async(gsr_ctx *c, void *host_frame) {
 
 GSR_API int gsr_peer_export_framebuffers(gsr_ctx *c, void *handles128) {
     if (!c || !handles128) return GSR_ERR_INVALID;
+    if (c->num_views > 1) return refuse_multiview("gsr_peer_export_framebuffers");
     if (!c->fb || !c->fb2 || c->fb_ext) { set_last_error("gsr_peer_export_framebuffers: call gsr_resize first (library-owned frames only)"); return GSR_ERR_STATE; }
     int rc = use_device(c->device);
     if (rc) return rc;
@@ -922,6 +1017,7 @@ GSR_API int gsr_peer_export_framebuffers(gsr_ctx *c, void *handles128) {
 
 GSR_API int gsr_peer_import_framebuffers(gsr_ctx *c, const void *handles128) {
     if (!c || !handles128) return GSR_ERR_INVALID;
+    if (c->num_views > 1) return refuse_multiview("gsr_peer_import_framebuffers");
     int rc = use_device(c->device);
     if (rc) return rc;
     cudaIpcMemHandle_t h[2];
@@ -950,6 +1046,7 @@ constexpr uint32_t GROUP_MAGIC = 0x47535247u;  // "GRSG"
 
 GSR_API int gsr_group_export(gsr_ctx *c, void *blob) {
     if (!c || !blob) return GSR_ERR_INVALID;
+    if (c->num_views > 1) return refuse_multiview("gsr_group_export");
     if (!c->fb || !c->fb2 || c->fb_ext) { set_last_error("gsr_group_export: call gsr_resize first (library-owned frames only)"); return GSR_ERR_STATE; }
     int rc = use_device(c->device);
     if (rc) return rc;
@@ -979,6 +1076,7 @@ GSR_API int gsr_group_export(gsr_ctx *c, void *blob) {
 GSR_API int gsr_group_attach(gsr_ctx *c, int32_t rank, int32_t world, const void *blobs) {
     if (!c || !blobs || world < 1 || world > GROUP_MAX || rank < 0 || rank >= world) { set_last_error("gsr_group_attach: need 0 <= rank < world <= %d", GROUP_MAX); return GSR_ERR_INVALID; }
     if (!c->grp.arena || !c->fb) { set_last_error("gsr_group_attach before gsr_group_export"); return GSR_ERR_STATE; }
+    if (c->num_views > 1) return refuse_multiview("gsr_group_attach");
     int rc = use_device(c->device);
     if (rc) return rc;
     group_detach(c);
@@ -1090,7 +1188,9 @@ GSR_API int gsr_pick(gsr_ctx *c, uint32_t tile_id, float heatmap_factor, float o
     if (rc) return rc;
     const uint32_t T = (uint32_t)(c->tiles_x * c->tiles_y);
     const uint32_t t0 = (uint32_t)(c->band_y0 * c->tiles_x), t1 = (uint32_t)(c->band_y1 * c->tiles_x);
-    if (tile_id < T && tile_id >= t0 && tile_id < t1 && (int)(tile_id / (uint32_t)c->tiles_x) % c->row_mod == c->row_rem) {
+    const bool owned = c->num_views > 1 ? tile_id < T * (uint32_t)c->num_views   // multiview: full frames, tile ids of all views
+                                        : (tile_id < T && tile_id >= t0 && tile_id < t1 && (int)(tile_id / (uint32_t)c->tiles_x) % c->row_mod == c->row_rem);
+    if (owned) {
         CompositeArgs ca;
         ca.records = c->records_cur; ca.values = c->vals_cur; ca.bounds = c->bounds; ca.out = framebuffer(c);
         ca.width = c->width; ca.height = c->height; ca.tiles_x = c->tiles_x;
@@ -1100,6 +1200,8 @@ GSR_API int gsr_pick(gsr_ctx *c, uint32_t tile_id, float heatmap_factor, float o
         ca.order = nullptr; ca.consumed = nullptr; ca.ctas_per_sm = 1; ca.sm_count = c->sm_count;
         ca.contract = (c->flags & GSR_FLAG_UNCONTRACTED_BLEND) ? 0 : 1;
         ca.trace = nullptr; ca.trace_count = nullptr; ca.trace_cap = 0;
+        ca.tiles_per_view = c->num_views > 1 ? (int32_t)T : 0;
+        ca.layer_stride = (uint64_t)c->width * c->height; ca.record_stride = 3ull * c->max_splats;
         for (int i = 0; i < 2; ++i)   // the re-dispatch rewrites the tile's pixels: not under a read-back in flight
             if (c->copied_valid[i]) GSR_CUDA_TRY(cudaStreamWaitEvent(c->stream, c->ev_copied[i], 0));
         GSR_CUDA_TRY(cudaMemsetAsync(c->pick_frame, 0, sizeof(FrameState), c->stream));
@@ -1179,6 +1281,7 @@ GSR_API int gsr_debug_compositor_config(gsr_ctx *c, int32_t ctas_per_sm, int32_t
 
 GSR_API int gsr_debug_pipeline(gsr_ctx *c, int32_t overlap) {
     if (!c) return GSR_ERR_INVALID;
+    if (c->num_views > 1 && overlap > 0) return refuse_multiview("gsr_debug_pipeline (overlap)");
     int rc = use_device(c->device);
     if (rc) return rc;
     GSR_CUDA_TRY(cudaStreamSynchronize(c->front_stream));
@@ -1210,13 +1313,13 @@ GSR_API int gsr_debug_copy(gsr_ctx *c, int which, void *dst, size_t bytes) {
     const void *src = nullptr;
     size_t avail = 0;
     switch (which) {
-        case GSR_BUF_RECORDS: src = c->records_cur; avail = sizeof(float4) * 3ull * c->max_splats; break;
+        case GSR_BUF_RECORDS: src = c->records_cur; avail = sizeof(float4) * 3ull * c->max_splats * (size_t)c->num_views; break;
         case GSR_BUF_KEYS: src = c->keys_cur; avail = sizeof(uint32_t) * c->capacity; break;
         case GSR_BUF_VALUES: src = c->vals_cur; avail = sizeof(uint32_t) * c->capacity; break;
-        case GSR_BUF_BOUNDS: src = c->bounds; avail = sizeof(uint2) * (size_t)c->tiles_x * c->tiles_y; break;
+        case GSR_BUF_BOUNDS: src = c->bounds; avail = sizeof(uint2) * frame_tiles(c); break;
         case GSR_BUF_KEYS_UNSORTED: src = c->unsorted_keys; avail = c->unsorted_keys ? sizeof(uint32_t) * c->capacity : 0; break;
         case GSR_BUF_VALUES_UNSORTED: src = c->unsorted_vals; avail = c->unsorted_vals ? sizeof(uint32_t) * c->capacity : 0; break;
-        case GSR_BUF_FRAMEBUFFER: src = framebuffer(c); avail = sizeof(float4) * (size_t)c->width * c->height; break;
+        case GSR_BUF_FRAMEBUFFER: src = framebuffer(c); avail = sizeof(float4) * frame_pixels(c); break;
         case GSR_BUF_COMPOSITOR_TRACE: src = c->trace; avail = c->trace ? sizeof(ulonglong4) * (size_t)c->trace_cap : 0; break;
         case GSR_BUF_COMPOSITOR_TRACE_COUNT: src = c->trace_count; avail = c->trace_count ? sizeof(uint32_t) : 0; break;
         default: set_last_error("gsr_debug_copy: unknown buffer %d", which); return GSR_ERR_INVALID;

@@ -963,6 +963,203 @@ __global__ void __launch_bounds__(PROJ_THREADS, GSR_PROJ_MIN_BLOCKS) projection_
     }
 }
 
+// ==============================================================================================================
+// Multiview frame (gsr_set_views): projection_kernel for K cameras at once.  Per warp, planes 0-2 arrive once (TMA) and the SH planes
+// at most once (bulk when enough lanes emit in ANY view, else per-lane gathers); per view the lane runs project_lane with that
+// view's constants, writes record words 0-1 into the view's table and parks its rect (n, x0|y0<<16, w|depth<<16) in shared memory
+// (registers stay at the single-view kernel's level whatever K is).  One chained scan runs over the per-splat SUM of the K counts;
+// a splat's pairs are emitted view-major, view v with tile ids v*T + tile -- so after the stable sort, view v's pairs are exactly
+// the single-view frame's pairs in the same order.
+constexpr size_t VIEW_STATE_BYTES = sizeof(uint32_t) * 3 * PROJ_THREADS;   // per view: n | x0,y0 | w,depth of every lane of the CTA
+
+__global__ void __launch_bounds__(PROJ_THREADS, GSR_PROJ_MIN_BLOCKS) projection_views_kernel(const __grid_constant__ ViewsArgs A) {
+#ifndef GSR_CPU_EMU
+    extern __shared__ __align__(128) unsigned char proj_smem[];
+#else
+    __shared__ __align__(128) unsigned char proj_smem[PROJ_SMEM_BYTES + GSR_MAX_VIEWS * VIEW_STATE_BYTES];
+#endif
+    __shared__ uint32_t s_bid;
+    __shared__ __align__(8) uint64_t s_bar[PROJ_WARPS][2];
+    __shared__ uint32_t s_wtotal[PROJ_WARPS];
+    __shared__ uint32_t s_count, s_ready, s_nvis;
+    __shared__ int32_t s_last;
+    __shared__ unsigned long long s_cta_base;
+
+    const ProjectionArgs &a = A.view[0];   // the view-independent fields
+    const int K = A.num_views;
+    const uint32_t T = A.tiles_per_view;
+    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
+    float4 *slab = reinterpret_cast<float4 *>(proj_smem + (size_t)warp * PROJ_SLAB_BYTES);  // [15][32]
+    uint32_t *vstate = reinterpret_cast<uint32_t *>(proj_smem + PROJ_SMEM_BYTES);           // [view][3][PROJ_THREADS]
+    if (lane == 0) {
+        mbar_init(&s_bar[warp][0], 1);
+        mbar_init(&s_bar[warp][1], 1);
+        fence_mbar_init();
+    }
+    if (tid == 0) {
+        s_bid = atomicAdd(&a.frame->proj_ticket, 1u);
+        s_count = 0u; s_ready = 0u; s_nvis = 0u; s_last = -1;
+    }
+    __syncthreads();
+    const uint32_t bid = s_bid;
+    const uint32_t id0 = (bid * PROJ_WARPS + warp) * 32u;
+    const uint32_t id = id0 + lane;
+
+    if (lane == 0) {
+        mbar_expect_tx(&s_bar[warp][0], 3u * 512u);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) bulk_g2s(slab + k * 32, a.soa + (uint64_t)k * a.plane_stride + id0, 512u, &s_bar[warp][0]);
+    }
+    const uint32_t gx = (uint32_t)((a.u.dims[0] + TILE - 1) / TILE);
+    mbar_wait(&s_bar[warp][0], 0);
+
+    // ---- phase 1, per view: cull + EWA + rect; record words 0-1; the rect to shared memory ----
+    uint32_t ntot = 0, any_mask = 0, nvis = 0;
+    int32_t last_tile = -1;   // in the concatenated tile-id space
+#pragma unroll 1
+    for (int v = 0; v < K; ++v) {
+        const ProjectionArgs &av = A.view[v];
+        uint32_t n = 0, xy = 0, wd = 0;
+        if (id < a.num_splats) {
+            LaneOut o;
+            if (project_lane<false>(av, slab[lane], slab[32 + lane], slab[64 + lane], o) && o.n) {
+                n = o.n; xy = o.x0 | (o.y0 << 16); wd = o.w | (o.depth << 16);
+                float4 *rec = av.records + (uint64_t)id * 3u;
+                rec[0] = o.r0; rec[1] = o.r1;
+            }
+            if (o.last_tile >= 0) last_tile = (int32_t)((uint32_t)v * T) + o.last_tile;
+        }
+        uint32_t *st = vstate + (size_t)v * 3u * PROJ_THREADS;
+        st[tid] = n; st[PROJ_THREADS + tid] = xy; st[2 * PROJ_THREADS + tid] = wd;
+        ntot += n;
+        const uint32_t m = __ballot_sync(0xffffffffu, n != 0u);
+        any_mask |= m;
+        nvis += (uint32_t)__popc(m);
+    }
+
+    // ---- scan of the per-splat totals; the closer publishes the CTA aggregate (as projection_kernel) ----
+    const uint32_t incl = warp_incl_scan_u32(ntot, lane);
+    const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+    const int32_t wl = __reduce_max_sync(0xffffffffu, last_tile);
+    bool closer = false;
+    uint32_t cta_total = 0;
+    if (lane == 0) {
+        s_wtotal[warp] = total;
+        if (nvis) atomicAdd(&s_nvis, nvis);
+        if (wl >= 0) atomicMax(&s_last, wl);
+        __threadfence_block();
+        closer = atomicAdd(&s_count, 1u) == PROJ_WARPS - 1;
+        if (closer) {
+            __threadfence_block();
+#pragma unroll
+            for (int w = 0; w < PROJ_WARPS; ++w) cta_total += ((volatile uint32_t *)s_wtotal)[w];
+            volatile unsigned long long *stl = a.lookback + bid;
+            *stl = (bid == 0 ? LB_PREFIX : LB_AGG) | (unsigned long long)cta_total;
+        }
+    }
+    closer = __shfl_sync(0xffffffffu, (int)closer, 0) != 0;
+    cta_total = __shfl_sync(0xffffffffu, cta_total, 0);
+
+    // ---- phase 2: the SH planes once for all views (bulk when enough lanes emit in any view), then colour + record word 2 per view ----
+    const bool bulk = (uint32_t)__popc(any_mask) >= (uint32_t)a.sh_bulk_min;
+    if (bulk && lane == 0) {
+        mbar_expect_tx(&s_bar[warp][1], 12u * 512u);
+#pragma unroll
+        for (int k = 3; k < NUM_PLANES; ++k) bulk_g2s(slab + k * 32, a.soa + (uint64_t)k * a.plane_stride + id0, 512u, &s_bar[warp][1]);
+    }
+    if (closer) {
+        const unsigned long long cta_base = lookback_exclusive(a.lookback, bid, (unsigned long long)cta_total, lane);
+        if (lane == 0) {
+            s_cta_base = cta_base;
+            __threadfence_block();
+            *(volatile uint32_t *)&s_ready = 1u;
+            const uint32_t nv = *(volatile uint32_t *)&s_nvis;
+            const int32_t lt = *(volatile int32_t *)&s_last;
+            if (nv) atomicAdd(&a.frame->visible, nv);
+            if (lt >= 0) atomicMax(&a.frame->last_tile_plus1, lt + 1);
+            if (bid == gridDim.x - 1) {
+                const unsigned long long m = cta_base + cta_total;
+                a.frame->dup_total = m;
+                a.frame->dup_sorted = m < (unsigned long long)a.capacity ? (uint32_t)m : a.capacity;
+                a.frame->overflow = m > (unsigned long long)a.capacity ? 1u : 0u;
+            }
+        }
+    }
+    if (bulk) mbar_wait(&s_bar[warp][1], 0);
+    if (any_mask & (1u << lane)) {
+        // the view-independent part of the record (opacity) and the view direction, with the operations of project_lane
+        const float4 pt = slab[lane], cb = slab[64 + lane];
+        const float ms = a.u.model_scale;
+        const float sp0 = pt.x * ms, sp1 = pt.y * ms, sp2 = pt.z * ms;
+        const float splat_time = a.u.time - pt.w;
+        const float tfl = ease_out_cubic(g_clamp(splat_time - 0.35f, 0.0f, 1.0f));
+        const float splat_opacity = cb.z * tfl * tfl;
+#pragma unroll 1
+        for (int v = 0; v < K; ++v) {
+            if (vstate[(size_t)v * 3u * PROJ_THREADS + tid] == 0u) continue;
+            const ProjectionArgs &av = A.view[v];
+            const float d0 = sp0 - av.u.camera_pos[0], d1 = sp1 - av.u.camera_pos[1], d2 = sp2 - av.u.camera_pos[2];
+            const float inv_len = 1.0f / sqrtf((d0 * d0 + d1 * d1) + d2 * d2);
+            float col[3];
+            if (bulk) sh_color<true>(slab + 3 * 32 + lane, 32, d0 * inv_len, d1 * inv_len, d2 * inv_len, col);
+            else sh_color<false>(a.soa + 3ull * a.plane_stride + id, a.plane_stride, d0 * inv_len, d1 * inv_len, d2 * inv_len, col);
+            av.records[(uint64_t)id * 3u + 2u] = make_float4(col[0], col[1], col[2], splat_opacity);
+        }
+    }
+
+    unsigned long long base = 0;
+    if (lane == 0) {
+        while (*(volatile uint32_t *)&s_ready == 0u) __nanosleep(100);
+        __threadfence_block();
+        base = *(volatile unsigned long long *)&s_cta_base;
+        for (uint32_t w = 0; w < warp; ++w) base += ((volatile uint32_t *)s_wtotal)[w];
+    }
+    base = __shfl_sync(0xffffffffu, base, 0);
+
+    // ---- emit, view-major per splat (same small / big rect rules as projection_kernel) ----
+    constexpr uint32_t EMIT_SMALL = 4;
+    uint32_t off = incl - ntot;
+#pragma unroll 1
+    for (int v = 0; v < K; ++v) {
+        const uint32_t *st = vstate + (size_t)v * 3u * PROJ_THREADS;
+        const uint32_t n = st[tid], x0u = st[PROJ_THREADS + tid] & 0xFFFFu, y0u = st[PROJ_THREADS + tid] >> 16;
+        const uint32_t wu = st[2 * PROJ_THREADS + tid] & 0xFFFFu, depth = st[2 * PROJ_THREADS + tid] >> 16;
+        const uint32_t tbase = (uint32_t)v * T;
+        if (n != 0u && n <= EMIT_SMALL) {
+            uint32_t x = x0u, y = y0u;
+            const uint32_t x1 = x0u + wu;
+#pragma unroll
+            for (uint32_t j = 0; j < EMIT_SMALL; ++j) {
+                if (j < n) {
+                    const unsigned long long g = base + off + j;
+                    if (g < (unsigned long long)a.capacity) {
+                        a.keys[g] = ((tbase + y * gx + x) << 16) | depth;
+                        a.values[g] = id;
+                    }
+                    if (++x == x1) { x = x0u; ++y; }
+                }
+            }
+        }
+        uint32_t big = __ballot_sync(0xffffffffu, n > EMIT_SMALL);
+        while (big) {
+            const int src = __ffs(big) - 1;
+            big &= big - 1u;
+            const uint32_t sn = __shfl_sync(0xffffffffu, n, src), soff = __shfl_sync(0xffffffffu, off, src);
+            const uint32_t sx0 = __shfl_sync(0xffffffffu, x0u, src), sy0 = __shfl_sync(0xffffffffu, y0u, src);
+            const uint32_t sw = __shfl_sync(0xffffffffu, wu, src), sdepth = __shfl_sync(0xffffffffu, depth, src);
+            for (uint32_t j = lane; j < sn; j += 32u) {
+                const uint32_t ry = j / sw, rx = j - ry * sw;
+                const unsigned long long g = base + soff + j;
+                if (g < (unsigned long long)a.capacity) {
+                    a.keys[g] = ((tbase + (sy0 + ry) * gx + sx0 + rx) << 16) | sdepth;
+                    a.values[g] = id0 + (uint32_t)src;
+                }
+            }
+        }
+        off += n;
+    }
+}
+
 }  // namespace
 
 uint32_t projection_num_blocks(uint32_t num_splats) { return (num_splats + PROJ_THREADS - 1) / PROJ_THREADS; }
@@ -979,6 +1176,17 @@ int preload_projection_kernels() {
     GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, projection_kernel));
     GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, projection_sharded_kernel));
     GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, projection_scatter_kernel));
+    GSR_CUDA_TRY(cudaFuncSetAttribute(projection_views_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)(PROJ_SMEM_BYTES + GSR_MAX_VIEWS * VIEW_STATE_BYTES)));
+    GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, projection_views_kernel));
+    return GSR_OK;
+}
+
+int launch_projection_views(const ViewsArgs &a, cudaStream_t stream) {
+    const uint32_t blocks = projection_num_blocks(a.view[0].num_splats);
+    if (blocks == 0) return GSR_OK;
+    projection_views_kernel<<<blocks, PROJ_THREADS, PROJ_SMEM_BYTES + (size_t)a.num_views * VIEW_STATE_BYTES, stream>>>(a);
+    GSR_CUDA_TRY(cudaGetLastError());
     return GSR_OK;
 }
 uint32_t projection_scatter_blocks(uint32_t count) { return count ? (count + PROJ_THREADS - 1) / PROJ_THREADS : 1u; }   // an empty slice still publishes its flags

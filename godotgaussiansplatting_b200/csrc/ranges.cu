@@ -66,6 +66,54 @@ __global__ void __launch_bounds__(256) tile_ranges_kernel(const uint32_t *__rest
     }
 }
 
+// Multiview frame: keys carry tile ids v*T + tile.  A view's list is the single-view frame's list with every index offset by the
+// view's first pair s_v, so the single-view rules apply per view: at a view boundary (key id-1 in view u, key id in a later view) the
+// plain end of u's last tile is NOT written; u's last key instead gets the tail rule of range_step, where "m - 1 >= 1" (the view has
+// at least two pairs) reads "key e-1 is in the same view"; the next view's first tile gets its start from the transition (a view
+// starting at pair 0 keeps start 0 from the clear, as the single-view frame's first tile does).
+__device__ __forceinline__ void view_tail(const uint32_t *__restrict__ keys, uint32_t e, uint32_t b, uint32_t T, uint2 *__restrict__ bounds, int quirks) {
+    if (quirks) {
+        if (b % T == T - 1u) {
+            if (e >= 1u && (keys[e - 1] >> 16) / T == b / T) bounds[b].y = e;
+        }
+    } else {
+        bounds[b].y = e + 1u;
+    }
+}
+
+__device__ __forceinline__ void range_step_views(const uint32_t *__restrict__ keys, uint32_t id, uint32_t a, uint32_t b, uint32_t m, uint2 *__restrict__ bounds,
+                                                 uint32_t T, int quirks) {
+    if (id > 0 && a != b) {
+        if (a / T == b / T) bounds[a].y = id;
+        else view_tail(keys, id - 1u, a, T, bounds, quirks);
+        bounds[b].x = id;
+    }
+    if (id == m - 1) view_tail(keys, id, b, T, bounds, quirks);
+}
+
+__global__ void __launch_bounds__(256) tile_ranges_views_kernel(const uint32_t *__restrict__ keys, const FrameState *__restrict__ frame,
+                                                                uint2 *__restrict__ bounds, uint32_t tiles_per_view, int quirks) {
+    const uint32_t m = frame->dup_sorted;
+    const uint32_t stride = gridDim.x * blockDim.x;
+    const uint32_t quads = m >> 2;
+    const uint4 *k4 = reinterpret_cast<const uint4 *>(keys);
+    for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < quads; q += stride) {
+        const uint4 k = __ldg(k4 + q);
+        const uint32_t id = q << 2;
+        const uint32_t prev = id ? __ldg(keys + id - 1) >> 16 : 0u;
+        const uint32_t t0 = k.x >> 16, t1 = k.y >> 16, t2 = k.z >> 16, t3 = k.w >> 16;
+        range_step_views(keys, id, prev, t0, m, bounds, tiles_per_view, quirks);
+        range_step_views(keys, id + 1, t0, t1, m, bounds, tiles_per_view, quirks);
+        range_step_views(keys, id + 2, t1, t2, m, bounds, tiles_per_view, quirks);
+        range_step_views(keys, id + 3, t2, t3, m, bounds, tiles_per_view, quirks);
+    }
+    for (uint32_t id = (quads << 2) + blockIdx.x * blockDim.x + threadIdx.x; id < m; id += stride) {
+        const uint32_t b = keys[id] >> 16;
+        const uint32_t a = id ? keys[id - 1] >> 16 : 0u;
+        range_step_views(keys, id, a, b, m, bounds, tiles_per_view, quirks);
+    }
+}
+
 // Fast sharded mode, after the ranks have all-reduced (MAX) their local last occupied tile: the rank that owns the
 // frame's last occupied tile L blanks it when L != T-1 -- in the reference that tile never gets its range end written
 // (gsplat_boundaries.glsl:47-49) and therefore renders nothing: rgb = 0, heat-map term (1 - t) = 0, alpha = 1.
@@ -152,6 +200,7 @@ int launch_frame_clear(FrameState *frame, unsigned long long *links, uint32_t n_
 int preload_ranges_kernels() {
     cudaFuncAttributes fa;
     GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, tile_ranges_kernel));
+    GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, tile_ranges_views_kernel));
     GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, band_fixup_kernel));
     GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, tile_order_kernel));
     GSR_CUDA_TRY(cudaFuncGetAttributes(&fa, frame_clear_kernel));
@@ -176,6 +225,13 @@ int launch_band_fixup(const int32_t *global_last_plus1, float4 *out, int32_t wid
 int launch_tile_ranges(const uint32_t *sorted_keys, const FrameState *frame, uint2 *bounds, uint32_t num_tiles, int quirks,
                        int sharded, int32_t *sync_word, int grid, cudaStream_t stream) {
     tile_ranges_kernel<<<grid, 256, 0, stream>>>(sorted_keys, frame, bounds, num_tiles, quirks, sharded, sync_word);
+    GSR_CUDA_TRY(cudaGetLastError());
+    return GSR_OK;
+}
+
+int launch_tile_ranges_views(const uint32_t *sorted_keys, const FrameState *frame, uint2 *bounds, uint32_t tiles_per_view, int quirks, int grid,
+                             cudaStream_t stream) {
+    tile_ranges_views_kernel<<<grid, 256, 0, stream>>>(sorted_keys, frame, bounds, tiles_per_view, quirks);
     GSR_CUDA_TRY(cudaGetLastError());
     return GSR_OK;
 }

@@ -69,6 +69,7 @@ class GaussianSplattingRasterizer:
         self.camera_transform = None
         self.camera_push_constants = None
         self._pinned = None
+        self._num_views = 1
 
     # ---- texture_size setter (rasterizer.gd:26-48) ----
     @property
@@ -218,6 +219,59 @@ class GaussianSplattingRasterizer:
         _lib.check(fn(self._ctx, vp.ctypes.data_as(C.POINTER(C.c_float)), u, float(self.should_enable_heatmap[0]), outp),
                    "gsr_render")
 
+    # ---- multiview (stereo / XR): K cameras of the same splats in one frame, K layers (include/gsr.h gsr_set_views) ----
+    @property
+    def num_views(self) -> int:
+        return self._num_views
+
+    def set_views(self, k: int) -> None:
+        if not self._ctx:
+            self.init_gpu(load=False)
+        _lib.check(_lib.lib().gsr_set_views(self._ctx, int(k)), "gsr_set_views")
+        self._num_views = int(k)
+        self._bind_texture()
+
+    def view_push_constants(self, camera: Camera3D, projection: np.ndarray | None = None) -> np.ndarray:
+        """The 128-byte push constant of one view (update_camera_matrices with basis_override applied); `projection` overrides the
+        camera's own perspective, e.g. with an off-axis camera.frustum for an XR eye."""
+        cam = np.asarray(camera.get_camera_transform(), dtype=np.float32).reshape(4, 4)
+        bo = self.basis_override
+        if np.array_equal(bo, np.eye(3, dtype=np.float32)):
+            view = cam.reshape(16)
+        else:
+            B = bo.T.astype(np.float32)
+            view = transform_to_projection((B @ cam[:3, :3].T).T.astype(np.float32), (B @ cam[3, :3]).astype(np.float32))
+        proj = camera.get_camera_projection() if projection is None else projection
+        return pack_camera_push_constants(view, np.asarray(proj, dtype=np.float32))
+
+    def rasterize_views(self, cameras, time: float | None = None, out_host: np.ndarray | None = None, asynchronous: bool = False,
+                        projections=None) -> None:
+        """rasterize() for K = num_views cameras at once: layer v of the frame is camera v's image, bit-identical to a single-view
+        rasterize() of that camera.  out_host: None, or (K, H, W, 4) float32 (synchronous: filled on return; asynchronous: page-locked,
+        filled once the copy stream is done, see sync())."""
+        cameras = list(cameras)
+        if len(cameras) != self._num_views:
+            raise ValueError(f"{len(cameras)} cameras for a context with {self._num_views} views (set_views)")
+        projections = list(projections) if projections is not None else [None] * len(cameras)
+        vp = np.ascontiguousarray(np.concatenate([self.view_push_constants(c, p) for c, p in zip(cameras, projections)]), dtype=np.float32)
+        t = self.ticks() if time is None else time
+        saved = self.camera
+        try:
+            ub = b""
+            for c in cameras:
+                self.camera = c
+                ub += self.uniforms_bytes(t)
+        finally:
+            self.camera = saved
+        L = _lib.lib()
+        outp = None if out_host is None else C.c_void_p(out_host.ctypes.data)
+        heat = float(self.should_enable_heatmap[0])
+        if asynchronous:
+            _lib.check(L.gsr_render_views_async(self._ctx, vp.ctypes.data_as(C.POINTER(C.c_float)), ub, heat, outp, _lib.GSR_OUT_RGBA32F),
+                       "gsr_render_views_async")
+        else:
+            _lib.check(L.gsr_render_views(self._ctx, vp.ctypes.data_as(C.POINTER(C.c_float)), ub, heat, outp), "gsr_render_views")
+
     def sync(self) -> None:
         _lib.check(_lib.lib().gsr_sync(self._ctx), "gsr_sync")
 
@@ -312,8 +366,9 @@ class GaussianSplattingRasterizer:
         return [buf[i] for i in range(got.value)]
 
     def read_framebuffer(self) -> np.ndarray:
+        """(H, W, 4) float32; (K, H, W, 4) in a context with K > 1 views."""
         w, h = self._texture_size
-        out = np.empty((h, w, 4), dtype=np.float32)
+        out = np.empty((h, w, 4) if self._num_views == 1 else (self._num_views, h, w, 4), dtype=np.float32)
         _lib.check(_lib.lib().gsr_debug_copy(self._ctx, _lib.GSR_BUF_FRAMEBUFFER, C.c_void_p(out.ctypes.data), out.nbytes),
                    "gsr_debug_copy")
         return out

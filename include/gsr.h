@@ -167,6 +167,35 @@ GSR_API int gsr_peer_import_framebuffers(gsr_ctx *ctx, const void *handles128);
 GSR_API int gsr_render(gsr_ctx *ctx, const float view_proj[32], const void *uniforms32, float heatmap_factor,
                        float *out_rgba32f_host);
 
+/* ---- multiview (stereo / XR): several cameras of one splat cloud in one frame.  No reference counterpart: an OpenXR host
+ *      (Godot's XRInterface: get_view_count(), get_transform_for_view(), get_projection_for_view()) renders every view of a frame
+ *      into one layer of a texture array.  The splats stay resident once; every splat is read once per frame and projected
+ *      for all K cameras; one sort and one compositor launch serve all views.
+ *      Layer v of a K-view frame is bit-identical to what gsr_render of camera v produces in a single-view context with the same
+ *      flags (incl. the Q10 tile-range quirks, applied per view, GSR_FLAG_FIXED_RANGES, GSR_FLAG_UNCONTRACTED_BLEND, heat-map and
+ *      load-in animation).
+ *      gsr_set_views(ctx, K), 1 <= K <= GSR_MAX_VIEWS (default 1): reallocates the K-layer frames, tile bounds and record tables.
+ *        GSR_ERR_INVALID (context unchanged) when K * tiles > 65536 (the sort key's 16-bit tile id: 4 views at 1920x1080, 2 at
+ *        3840x2160); GSR_ERR_STATE in a context with a shard group, peer frames, a band or row interleave, or overlap on -- and those
+ *        calls return GSR_ERR_STATE while K > 1.  gsr_resize applies the same K * tiles check.
+ *      In a K > 1 context: gsr_render / gsr_render_async* return GSR_ERR_STATE (use the calls below); the frame is K layers of
+ *        W*H RGBA32F pixels, layer v at pixel offset v*W*H (a VK_IMAGE_VIEW_TYPE_2D_ARRAY image of K layers); gsr_framebuffer_device_ptr
+ *        is layer 0, gsr_set_framebuffer_external needs K layers, gsr_present_device / gsr_readback_async convert or copy all K
+ *        layers; gsr_pick takes tile ids in [0, K*T) (view = tile_id / T); gsr_get_stats / gsr_get_frame_history report M, V and C
+ *        summed over the views and last_tile in that concatenated id space; the gsr_debug_copy taps cover all views (K*T bounds,
+ *        K record tables of max_splats records, the K-layer frame).
+ *      view_proj: K push constants of 32 floats (any projection, incl. the asymmetric per-eye frusta of XR).
+ *      uniforms:  K uniform blocks of 32 bytes; they must agree on model_scale, width, height and time (else GSR_ERR_INVALID) --
+ *                 only camera_pos differs between views. ---- */
+#define GSR_MAX_VIEWS 4
+GSR_API int gsr_set_views(gsr_ctx *ctx, int32_t num_views);
+/* out_rgba32f_host: NULL (frame stays on the device) or K*W*H*4 floats, layer-major; synchronous like gsr_render. */
+GSR_API int gsr_render_views(gsr_ctx *ctx, const float *view_proj /* K x 32 */, const void *uniforms /* K x 32 B */,
+                             float heatmap_factor, float *out_rgba32f_host);
+/* Pipelined read-back of all K layers (gsr_render_async_fmt): pinned_host holds K x gsr_output_bytes(format, W, H) bytes. */
+GSR_API int gsr_render_views_async(gsr_ctx *ctx, const float *view_proj, const void *uniforms, float heatmap_factor,
+                                   void *pinned_host, int32_t format);
+
 /* Pipelined host read-back: enqueue the frame and an asynchronous device->host copy into `pinned_host` (page-locked
  * memory; with pageable memory the copy degrades to a synchronous one).  Frames alternate between two internal
  * framebuffers and the copy runs on a separate stream, so the read-back of frame i overlaps the kernels of frame i+1.
